@@ -3,7 +3,7 @@
 log marginal likelihood in FP64 at N = 60 000, D = 784 (MNIST-shaped), one "step" = one full evaluation of
 SPR.loss (spax/models.py:93-98) on one batch of inputs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N = 1 runs the single-GPU fused C-ABI call; N > 1 (under torchrun, one rank per GPU) runs the block-cyclic
 distributed driver over NCCL on the SAME fixed problem (strong scaling).  Prints ONE JSON line on rank 0.
@@ -38,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the bench writes nothing into the tree it runs from (it may be read-only)
 
 METRIC = "NNGP Gram+Cholesky+Student-t LML time & FP64 TFLOP/s, N=60k, 1/2/4/8 B200"
 UNIT = "TFLOP/s"
@@ -137,6 +138,14 @@ def host_threads():
     return max(n, 1), os.cpu_count()
 
 
+def dump_outputs(path, arrays):
+    """--dump-outputs: what the timed call returned in its last step, one PATH/<name>.npy per array in float64, so
+    that two builds run on the same seeded inputs can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def _c3_golden(n, d):
     """tests/golden/c3_full.json: losses recorded for the exact bench workload (N, D, seed 10, reference defaults)"""
     path = os.path.join(ROOT, "tests", "golden", "c3_full.json")
@@ -170,25 +179,19 @@ def run_reference(args):
     n, d = min(args.n, CPU_SAMPLE_N), args.d
     x, y = make_inputs(args.n, d)
     x, y = x[:n], y[:n]                                  # the SAME rows the GPU arm's same_config_check evaluates
-    # W warm-up + K timed steps, bounded to ~4 min of wall clock in total: the first warm-up step calibrates, the
-    # remaining warm-ups and the number of timed steps shrink if (W + K) steps would not fit (reported as `steps`)
-    budget_s = 240.0
-    t_first, _ = cpu_port_step(x, y)
-    fit = max(1, int(budget_s / max(t_first, 1e-3)) - 1)
-    n_warm = max(0, min(args.warmup - 1, fit - 1))
-    for _ in range(n_warm):
+    for _ in range(args.warmup):
         cpu_port_step(x, y)
-    k_timed = max(1, min(args.steps, fit - n_warm))
-    res = [cpu_port_step(x, y) for _ in range(k_timed)]
+    res = [cpu_port_step(x, y) for _ in range(args.steps)]
     times, loss = [r[0] for r in res], float(res[-1][1])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"loss": loss})
     t = float(np.mean(times))
     val = lml_flops(n, d) / t * 1e-12
     blas_threads, cores = host_threads()
     sample = (f"first {n} of the {args.n} rows of the same synthetic workload (D={d}, L=3 ReLU, Student-t LML); "
               f"the full N would need ~{(args.n / n) ** 3 * t / 60:.0f} min of CPU time")
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
-            "steps": k_timed, "warmup": n_warm + 1, "steps_requested": args.steps, "warmup_requested": args.warmup,
-            "ms_per_step": t * 1e3, "higher_is_better": True,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": t * 1e3, "higher_is_better": True,
             "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": workload_config(args.n, d), "loss_on_sample": loss,
             "cpu_baseline": {"value": val, "unit": UNIT, "cores": blas_threads, "host_cpus": cores, "kind": "port",
@@ -251,6 +254,8 @@ def run_ours(args):
         e1.record()
         barrier()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": out[0].cpu().numpy(), "info": out[1].cpu().numpy()})
     launches = int(lib.smnngp_instr_launches())
     import ctypes as C
     upd_ms, upd_flops = C.c_double(0), C.c_double(0)
@@ -453,7 +458,12 @@ def main():
     ap.add_argument("--features", dest="d", type=int, default=784, help="D (input features)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-grad", action="store_true", help="skip the extra value+gradient measurement (N = 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float64): "
+                         "out = [log p(y), loss, sum log L_ii, ||L^-1 y||^2] and info (reference arm: loss)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -5,13 +5,15 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_one_json_line():
+def test_reference_arm_prints_one_json_line(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--rows", "1500",
-                        "--features", "16", "--steps", "1", "--warmup", "0"], capture_output=True, text=True,
-                       timeout=300, cwd=ROOT)
+                        "--features", "16", "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -21,6 +23,15 @@ def test_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["sample"]
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0
     assert "workload" in d["config"]
+    assert d["steps"] == 2 and d["warmup"] == 0
+    loss = np.load(tmp_path / "loss.npy")
+    assert loss.dtype == np.float64 and loss.shape == () and float(loss) == d["loss_on_sample"]
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode != 0 and "--steps" in r.stderr
 
 
 def test_reference_arm_other_ranks_exit_quietly():
