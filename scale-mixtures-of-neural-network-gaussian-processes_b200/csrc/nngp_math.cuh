@@ -28,7 +28,10 @@ __device__ __forceinline__ double encode_var(double u, int act) {
 // (rsqrt.approx / rcp.approx on the double directly) + Newton steps, one division, an 11-term minimax
 // polynomial for atan on |z| <= tan(pi/8) (fitted in 60-digit arithmetic, relative error 2.2e-16).
 // Accuracy of phi: <= 2.5e-16 * sqrt(u1 u2) absolute (checked against 50-digit mpmath), i.e. the same as the
-// libm formulation.  Magnitudes below 1e-30 are treated as zero (inputs are O(1) standardised features).
+// libm formulation, for layer variances with 1e-260 <= u1 u2 <= 1e300.  u is a layer variance, not an input: a deep
+// ReLU stack halves it at every layer, small weights or inputs in small units shrink it further, and the radicand
+// u1 u2 - k^2 is of the order of u^2.  The seeds are floored at 1e-300, where rsqrt / rcp still return normal
+// doubles; a radicand below the floor belongs to a pair with s < 1e-150, which phi ~ sqrt(u1 u2) cannot resolve.
 __device__ __forceinline__ double rsqrt_seed(double x) {
   double y;
   asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
@@ -40,7 +43,7 @@ __device__ __forceinline__ double rcp_seed(double x) {
   return y;
 }
 __device__ __forceinline__ double sqrt_nobranch(double x) {          // x >= 0
-  const double y = rsqrt_seed(fmax(x, 1e-30));
+  const double y = rsqrt_seed(fmax(x, 1e-300));
   double g = x * y, h = 0.5 * y;
   double r = fma(-g, h, 0.5);
   g = fma(g, r, g); h = fma(h, r, h);
@@ -48,7 +51,7 @@ __device__ __forceinline__ double sqrt_nobranch(double x) {          // x >= 0
   g = fma(g, r, g); h = fma(h, r, h);
   return fma(fma(-g, g, x), h, g);
 }
-__device__ __forceinline__ double div_nobranch(double n, double d) {  // d >= 1e-30
+__device__ __forceinline__ double div_nobranch(double n, double d) {  // d >= 1e-300
   double y = rcp_seed(d);
   double e = fma(-d, y, 1.0);
   y = fma(y, e, y);
@@ -64,7 +67,7 @@ __device__ __forceinline__ double phi_relu_parts(double k, double t1, double t2,
   const double ax = fabs(k);
   const bool swap = s > ax;
   const double num = swap ? ax : s;
-  const double den = fmax(swap ? s : ax, 1e-30);
+  const double den = fmax(swap ? s : ax, 1e-300);
   const bool hi = num > 0.41421356237309503 * den;                   // tan(pi/8): atan(r) = pi/4 + atan((r-1)/(r+1))
   const double z = div_nobranch(hi ? num - den : num, hi ? num + den : den);
   const double w = z * z;
