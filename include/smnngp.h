@@ -138,6 +138,20 @@ int smnngp_grid_point_f64(void* stream, const double* K0dd, int64_t ld0, const d
                           const double* q_d, const double* q_t, const double* y, int64_t N, int64_t T, int n_hidden,
                           int act, int arch, const double* hp_dev, void* workspace, size_t workspace_bytes,
                           double* mean_out, double* var_out, double* out_dev, int* info_dev);
+/* grid_batch  G points in ONE launch for N <= 4096 (the reference's UCI sizes), where a single point leaves the GPU
+ *             nearly idle: a CTA evaluates a whole point in its own slot of the workspace and walks the points with a
+ *             static stride.  Inputs as grid_point; hp_dev [G][6]; mean_out [G][T], var_out [G][T], out_dev [G][2] and
+ *             info_dev [G]: row g is what grid_point returns for hp_dev + 6 g (NaN outputs when a factorisation fails),
+ *             and no point affects another: a point's outputs are the same bits in any batch, order or slot count.
+ *             The slot count (points in flight) is workspace_bytes / smnngp_grid_batch_workspace_bytes(.., 1); each
+ *             slot holds the (N + T + 1) x N trapezoid and the layer tables.  Fewer than one slot: SMNNGP_EWORKSPACE;
+ *             N > 4096, T < 1, G < 1, a null pointer, ld0 or ld0t < N or an invalid stack: SMNNGP_EINVAL, both before
+ *             anything is enqueued.  Enqueue-only (one kernel launch), no allocation, graph-capturable. */
+size_t smnngp_grid_batch_workspace_bytes(int64_t N, int64_t T, int n_hidden, int arch, int64_t slots);
+int smnngp_grid_batch_f64(void* stream, const double* K0dd, int64_t ld0, const double* K0td, int64_t ld0t,
+                          const double* q_d, const double* q_t, const double* y, int64_t N, int64_t T, int64_t G,
+                          int n_hidden, int act, int arch, const double* hp_dev, void* workspace,
+                          size_t workspace_bytes, double* mean_out, double* var_out, double* out_dev, int* info_dev);
 
 /* ---- posterior draw stage of the classification / ensemble configuration (SURVEY section 8f, row N2).
  * mean [T, C]; var [T] (shared by the classes, var_per_class = 0) or [C, T] (var_per_class = 1); kind STUDENT_T:

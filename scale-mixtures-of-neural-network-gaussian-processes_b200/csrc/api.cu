@@ -618,6 +618,54 @@ int smnngp_grid_point_f64(void* stream, const double* K0dd, int64_t ld0, const d
   return SMNNGP_OK;
 }
 
+// the whole grid in one launch (grid_batch.cu): one slot per point in flight, the trapezoid first, then the tables
+namespace {
+size_t carve_grid_slot(GridBatchParams& p, long long N, long long T, int n_act) {
+  const size_t na = (size_t)(n_act > 0 ? n_act : 1);
+  Carver c(nullptr);
+  p.lda = round_up(N, 16);
+  c.take<double>((size_t)(N + T + 1) * p.lda);
+  p.off_tab = (long long)(c.total() / 8);
+  c.take<double>(na * N);
+  p.off_q = (long long)(c.total() / 8);
+  c.take<double>(N);
+  p.off_tab_t = (long long)(c.total() / 8);
+  c.take<double>(na * T);
+  p.off_q_t = (long long)(c.total() / 8);
+  c.take<double>(T);
+  p.slot_bytes = (long long)c.total();
+  return c.total();
+}
+}  // namespace
+
+size_t smnngp_grid_batch_workspace_bytes(int64_t N, int64_t T, int n_hidden, int arch, int64_t slots) {
+  GridBatchParams p{};
+  return (size_t)(slots > 0 ? slots : 0) * carve_grid_slot(p, N, T, n_act_applications(n_hidden, arch));
+}
+
+int smnngp_grid_batch_f64(void* stream, const double* K0dd, int64_t ld0, const double* K0td, int64_t ld0t,
+                          const double* q_d, const double* q_t, const double* y, int64_t N, int64_t T, int64_t G,
+                          int n_hidden, int act, int arch, const double* hp_dev, void* workspace,
+                          size_t workspace_bytes, double* mean_out, double* var_out, double* out_dev, int* info_dev) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  if (!K0dd || !K0td || !q_d || !q_t || !y || !hp_dev || !mean_out || !var_out || !out_dev || !info_dev || N < 1 ||
+      N > GRID_BATCH_MAX_N || T < 1 || G < 1 || ld0 < N || ld0t < N || !valid_stack(n_hidden, act, arch) ||
+      N + T + 1 > INT32_MAX || G > INT32_MAX)
+    return fail(SMNNGP_EINVAL, "smnngp_grid_batch_f64: invalid argument");
+  GridBatchParams p{};
+  const size_t slot_bytes = carve_grid_slot(p, N, T, n_act_applications(n_hidden, arch));
+  const long long slots = workspace ? (long long)(workspace_bytes / slot_bytes) : 0;
+  if (slots < 1) return fail(SMNNGP_EWORKSPACE, "smnngp_grid_batch_f64: workspace holds no slot");
+  p.K0dd = K0dd; p.K0td = K0td; p.q_d = q_d; p.q_t = q_t; p.y = y; p.hp = hp_dev;
+  p.ld0 = ld0; p.ld0t = ld0t;
+  p.N = (int)N; p.T = (int)T; p.G = (int)G; p.n_hidden = n_hidden; p.arch = arch;
+  p.ws = static_cast<char*>(workspace);
+  p.mean = mean_out; p.var = var_out; p.out = out_dev; p.info = info_dev;
+  CU(launch_grid_batch(s, p, act, slots));
+  return SMNNGP_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // host-buffer entry points
 // ---------------------------------------------------------------------------------------------------------

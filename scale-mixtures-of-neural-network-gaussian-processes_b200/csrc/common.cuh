@@ -68,6 +68,20 @@ __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
+// fixed-order sum over a CTA of NT threads (red: NT / 32 doubles of shared memory); every thread gets the result
+template <int NT>
+__device__ __forceinline__ double block_sum(double v, double* red) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();
+  if (lane == 0) red[warp] = v;
+  __syncthreads();
+  double s = 0.0;
+  for (int k = 0; k < NT / 32; k++) s += red[k];
+  return s;
+}
+
 // Linear tile id -> (ti, tj).  lower != 0: only tiles that contain an element with col <= row (the region
 // starts on the diagonal; rows may extend past the column count = trapezoid).  With BM = Q*BN row tile r owns
 // min(ntn, Q*r + Q) column tiles.  ntn = number of column tiles.

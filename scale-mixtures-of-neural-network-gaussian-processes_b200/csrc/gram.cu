@@ -12,30 +12,6 @@ namespace smnngp {
 
 namespace {
 
-// per-row layer tables from the input variance q0 = ||x||^2 / D.  hp == nullptr: unit scalars (w = v = 1, b = 0)
-__device__ __forceinline__ void fill_row_tables(double q, int row, int n_hidden, int act, int arch,
-                                                const double* __restrict__ hp, double* __restrict__ tab,
-                                                long long tab_ld, double* __restrict__ qfin) {
-  const double w2 = hp ? hp[HP_W] * hp[HP_W] : 1.0, b2 = hp ? hp[HP_B] * hp[HP_B] : 0.0,
-               v2 = hp ? hp[HP_V] * hp[HP_V] : 1.0;
-  if (arch == ARCH_MLP) {
-    for (int a = 0; a < n_hidden; a++) {
-      double u = w2 * q + b2;
-      tab[a * tab_ld + row] = encode_var(u, act);
-      q = act_diag(u, act);
-    }
-  } else {
-    double u = w2 * q + b2;
-    for (int a = 0; a < n_hidden; a++) {
-      tab[a * tab_ld + row] = encode_var(u, act);
-      u = u + (w2 * act_diag(u, act) + b2);
-    }
-    tab[(long long)n_hidden * tab_ld + row] = encode_var(u, act);
-    q = act_diag(u, act);
-  }
-  qfin[row] = v2 * q;
-}
-
 __global__ void qtable_kernel(const double* __restrict__ X, long long ldx, int N, int D, int n_hidden, int act,
                               int arch, const double* __restrict__ hp, double* __restrict__ tab,
                               long long tab_ld, double* __restrict__ qfin) {
@@ -146,10 +122,7 @@ __device__ __forceinline__ void gram_epilogue(const GramParams& p, double (&acc)
           for (int ni = 0; ni < NI; ni++)
 #pragma unroll
             for (int e = 0; e < 2; e++) {
-              double k = acc[u][ni][e];
-              if (!resnet) k = w2 * k + b2;
-              const double ph = phi<ACT>(k, tr[u], tc[ni][e]);
-              res[u][ni][e] = plain ? ph : k + (w2 * ph + b2);
+              res[u][ni][e] = layer_step<ACT>(acc[u][ni][e], tr[u], tc[ni][e], w2, b2, resnet, plain);
             }
 #pragma unroll
         for (int mi = 0; mi < MI - RU; mi++) {

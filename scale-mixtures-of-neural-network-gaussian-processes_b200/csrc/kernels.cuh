@@ -19,7 +19,7 @@ int* lookahead_reserve();
 // diagnostic: when non-null, thread 0 of the diagonal-block kernel stores clock64() at its phase boundaries
 long long*& potf2_clock_buffer();
 
-inline int n_act_applications(int n_hidden, int arch) { return arch == ARCH_RESNET ? n_hidden + 1 : n_hidden; }
+__host__ __device__ inline int n_act_applications(int n_hidden, int arch) { return arch == ARCH_RESNET ? n_hidden + 1 : n_hidden; }
 
 struct GramParams {
   const double* X1;   // [N, D] rows of the output
@@ -135,6 +135,22 @@ cudaError_t launch_test_nll_finalize(cudaStream_t s, const double* mean, const d
                                      int kind, const double* quad2, const int* info, double* logp,
                                      double* nll_out);
 cudaError_t launch_fill_nan_if_bad(cudaStream_t s, const int* info, double* buf, long long n);
+
+// ---- batched grid search (grid_batch.cu) ---------------------------------------------------------------------
+constexpr int GRID_BATCH_MAX_N = 4096;
+struct GridBatchParams {
+  const double *K0dd, *K0td, *q_d, *q_t, *y;   // cached bases (smnngp_grid_base_f64) and the targets
+  const double* hp;                            // [G][HP_COUNT]
+  long long ld0, ld0t;
+  int N, T, G, n_hidden, arch;
+  char* ws;                                    // slot k at ws + k * slot_bytes
+  long long slot_bytes, lda;                   // lda: row stride of a slot's (N + T + 1)-row trapezoid
+  long long off_tab, off_q, off_tab_t, off_q_t;   // layer tables inside a slot (doubles from its start)
+  double *mean, *var, *out;                    // [G][T], [G][T], [G][2]
+  int* info;                                   // [G]
+};
+// one persistent launch: min(slots, G) CTAs, each owns one slot and evaluates points blockIdx.x, + gridDim.x, ...
+cudaError_t launch_grid_batch(cudaStream_t s, const GridBatchParams& p, int act, long long slots);
 
 // ---- gradient of the log marginal likelihood (grad.cu) -------------------------------------------------------
 // tab3 [3][n_act][tab_ld]: encoded marginal variances + the two dual planes the gradient epilogue needs

@@ -2,7 +2,7 @@
 // semantics): diagonal maps, the branch-free ReLU arc-cosine step and the erf step, plus their partial
 // derivatives (used by the gradient pass, grad.cu).
 #pragma once
-#include "common.cuh"
+#include "kernels.cuh"
 
 namespace smnngp {
 
@@ -105,6 +105,40 @@ __device__ __forceinline__ double phi(double k, double t1, double t2) {
     x = fmin(fmax(x, -1.0), 1.0);
     return kTwoOverPi * asin(x);
   }
+}
+
+// per-row layer tables from the input variance q0 = ||x||^2 / D.  hp == nullptr: unit scalars (w = v = 1, b = 0)
+__device__ __forceinline__ void fill_row_tables(double q, int row, int n_hidden, int act, int arch,
+                                                const double* __restrict__ hp, double* __restrict__ tab,
+                                                long long tab_ld, double* __restrict__ qfin) {
+  const double w2 = hp ? hp[HP_W] * hp[HP_W] : 1.0, b2 = hp ? hp[HP_B] * hp[HP_B] : 0.0,
+               v2 = hp ? hp[HP_V] * hp[HP_V] : 1.0;
+  if (arch == ARCH_MLP) {
+    for (int a = 0; a < n_hidden; a++) {
+      double u = w2 * q + b2;
+      tab[a * tab_ld + row] = encode_var(u, act);
+      q = act_diag(u, act);
+    }
+  } else {
+    double u = w2 * q + b2;
+    for (int a = 0; a < n_hidden; a++) {
+      tab[a * tab_ld + row] = encode_var(u, act);
+      u = u + (w2 * act_diag(u, act) + b2);
+    }
+    tab[(long long)n_hidden * tab_ld + row] = encode_var(u, act);
+    q = act_diag(u, act);
+  }
+  qfin[row] = v2 * q;
+}
+
+// One layer of the recursion on one kernel entry k given the encoded marginals of its row and column: an MLP layer
+// (Dense then the nonlinearity), a dense-resnet block (k + Dense(phi(k))), or the resnet's trailing activation (plain).
+template <int ACT>
+__device__ __forceinline__ double layer_step(double k, double tr, double tc, double w2, double b2, bool resnet,
+                                             bool plain) {
+  if (!resnet) k = w2 * k + b2;
+  const double ph = phi<ACT>(k, tr, tc);
+  return plain ? ph : k + (w2 * ph + b2);
 }
 
 }  // namespace smnngp

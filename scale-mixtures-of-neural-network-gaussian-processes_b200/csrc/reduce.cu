@@ -12,19 +12,6 @@ namespace {
 constexpr double kPi = 3.14159265358979323846;
 __device__ __forceinline__ double qnan() { return __longlong_as_double(0x7ff8000000000000ll); }
 
-template <int NT>
-__device__ __forceinline__ double block_sum(double v, double* red) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  __syncthreads();
-  if (lane == 0) red[warp] = v;
-  __syncthreads();
-  double s = 0.0;
-  for (int k = 0; k < NT / 32; k++) s += red[k];
-  return s;
-}
-
 __global__ void sumsq_kernel(const double* __restrict__ z, long long n, double* __restrict__ out) {
   __shared__ double red[32];
   double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;

@@ -406,6 +406,18 @@ def grid_point(x, y, x_test, *, spec: StackSpec, hp):
     return mean[:, 0], var, 2.0 * out[2], out[3], torch.maximum(info1, info2)
 
 
+GRID_BATCH_MAX_N = 4096
+
+
+def _batch_wins(n, g):
+    """Whether ``GridSearch.points`` evaluates G points of N training rows in one batched launch rather than one
+    point after the other.  Up to the resident slots the batch costs what one CTA needs for one point; that is
+    3.2, 8.9, 38 and 130 times a ``point`` call at N = 404, 824, 2048 and 4096 (profiles/r03_grid_batch.jsonl, B200 at
+    1000 W), ~3.2 (N / 404)^1.6.  Past the slots the batch runs in waves of at least 148 points, which still beats the
+    loop wherever one wave does."""
+    return n <= GRID_BATCH_MAX_N and g >= 3.2 * (n / 404.0) ** 1.6
+
+
 class GridSearch:
     """The reference's hyper-parameter grid search (experiments/regression/find.py:134-199) with the base Gram cached:
     X.X^T / D, Xt.X^T / D and the input variances are computed once; every ``point(hp)`` is recursion-only passes over
@@ -447,6 +459,35 @@ class GridSearch:
                                                 _p(hp), _p(ws), ws_bytes, _p(mean), _p(var), _p(out), _p(info))
         _lib.check(rc, "grid_point")
         return mean, var, 2.0 * out[0], out[1], info
+
+    def points(self, hps):
+        """Every row of ``hps`` [G, 6] (device operand rows, e.g. ``torch.stack`` of make_hp) at once:
+        (mean [G, T], var [G, T], logdet [G], quad [G], info [G]), row g what ``point(hps[g])`` returns.  Where one
+        launch for the whole grid is faster (``_batch_wins``) a CTA evaluates each point in its own workspace slot
+        (smnngp_grid_batch_f64); elsewhere, and always for N > 4096, the points run one after the other."""
+        dev = self.y.device
+        hps = _f64(hps, dev)
+        if hps.ndim != 2 or hps.shape[1] != 6:
+            raise ValueError("hps must be [G, 6]")
+        g = hps.shape[0]
+        if not _batch_wins(self.n, g):
+            rows = [self.point(hps[i]) for i in range(g)]
+            return tuple(torch.stack([r[k] for r in rows]) for k in range(4)) + (torch.cat([r[4] for r in rows]),)
+        nh, act, arch = self.spec.ids()
+        mean = torch.empty((g, self.t), dtype=torch.float64, device=dev)
+        var = torch.empty((g, self.t), dtype=torch.float64, device=dev)
+        out = torch.empty((g, 2), dtype=torch.float64, device=dev)
+        info = torch.empty(g, dtype=torch.int32, device=dev)
+        # every slot a CTA the device keeps resident (grid_batch_kernel: two per SM); more would only wait
+        slots = min(g, 2 * torch.cuda.get_device_properties(dev).multi_processor_count)
+        ws_bytes = self.lib.smnngp_grid_batch_workspace_bytes(self.n, self.t, nh, arch, slots)
+        with torch.cuda.device(dev):
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            rc = self.lib.smnngp_grid_batch_f64(_stream(dev), _p(self.k0dd), self.ld0, _p(self.k0td), self.ld0,
+                                                _p(self.q_d), _p(self.q_t), _p(self.y), self.n, self.t, g, nh, act,
+                                                arch, _p(hps), _p(ws), ws_bytes, _p(mean), _p(var), _p(out), _p(info))
+        _lib.check(rc, "grid_batch")
+        return mean, var, 2.0 * out[:, 0], out[:, 1], info
 
 
     def sweep_eps(self, eps_list, hp, group=None):
