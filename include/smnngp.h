@@ -152,6 +152,22 @@ int smnngp_grid_batch_f64(void* stream, const double* K0dd, int64_t ld0, const d
                           const double* q_d, const double* q_t, const double* y, int64_t N, int64_t T, int64_t G,
                           int n_hidden, int act, int arch, const double* hp_dev, void* workspace,
                           size_t workspace_bytes, double* mean_out, double* var_out, double* out_dev, int* info_dev);
+/* lml_grad_batch  SPR.loss and its gradient at G points in ONE launch for N <= 4096 (multi-start training, gradient
+ *             refinement of a grid search).  K0dd / ld0 / q_d are the bases of grid_base with T = 0, y [N] the targets;
+ *             hp_dev [G][6]; kind as smnngp_lml_grad_f64 (absolute regulariser K + eps I).  out_dev [G][4], grad_dev
+ *             [G][6] and info_dev [G]: row g is what smnngp_lml_grad_f64 returns for hp_dev + 6 g, up to rounding
+ *             (same matrix, different blocking).  When a factorisation fails all of out_dev[g] and grad_dev[g] are
+ *             NaN and info_dev[g] = 1 + the first bad pivot.  No point affects another: a point's outputs are the
+ *             same bits in any batch, order or slot count.  The slot count is workspace_bytes /
+ *             smnngp_lml_grad_batch_workspace_bytes(.., 1); each slot holds the (2N + 1) x N trapezoid A | y^T | I,
+ *             the dual layer tables and A^-1 y.  Fewer than one slot: SMNNGP_EWORKSPACE; N < 1, N > 4096, G < 1, a
+ *             null pointer, ld0 < N, an invalid stack or kind: SMNNGP_EINVAL, both before anything is enqueued.
+ *             Enqueue-only (one kernel launch), no allocation, graph-capturable. */
+size_t smnngp_lml_grad_batch_workspace_bytes(int64_t N, int n_hidden, int arch, int64_t slots);
+int smnngp_lml_grad_batch_f64(void* stream, const double* K0dd, int64_t ld0, const double* q_d, const double* y,
+                              int64_t N, int64_t G, int n_hidden, int act, int arch, const double* hp_dev, int kind,
+                              void* workspace, size_t workspace_bytes, double* out_dev, double* grad_dev,
+                              int* info_dev);
 
 /* ---- posterior draw stage of the classification / ensemble configuration (SURVEY section 8f, row N2).
  * mean [T, C]; var [T] (shared by the classes, var_per_class = 0) or [C, T] (var_per_class = 1); kind STUDENT_T:

@@ -666,6 +666,49 @@ int smnngp_grid_batch_f64(void* stream, const double* K0dd, int64_t ld0, const d
   return SMNNGP_OK;
 }
 
+// loss and gradient at every point in one launch (grad_batch.cu): the trapezoid A | y^T | I, then the tables and A^-1 y
+namespace {
+size_t carve_grad_slot(GradBatchParams& p, long long N, int n_act) {
+  const size_t na = (size_t)(n_act > 0 ? n_act : 1);
+  Carver c(nullptr);
+  p.lda = round_up(N, 16);
+  c.take<double>((size_t)(2 * N + 1) * p.lda);
+  p.off_tab3 = (long long)(c.total() / 8);
+  c.take<double>(3 * na * N);
+  p.off_alpha = (long long)(c.total() / 8);
+  c.take<double>(N);
+  p.slot_bytes = (long long)c.total();
+  return c.total();
+}
+}  // namespace
+
+size_t smnngp_lml_grad_batch_workspace_bytes(int64_t N, int n_hidden, int arch, int64_t slots) {
+  GradBatchParams p{};
+  return (size_t)(slots > 0 ? slots : 0) * carve_grad_slot(p, N, n_act_applications(n_hidden, arch));
+}
+
+int smnngp_lml_grad_batch_f64(void* stream, const double* K0dd, int64_t ld0, const double* q_d, const double* y,
+                              int64_t N, int64_t G, int n_hidden, int act, int arch, const double* hp_dev, int kind,
+                              void* workspace, size_t workspace_bytes, double* out_dev, double* grad_dev,
+                              int* info_dev) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  if (!K0dd || !q_d || !y || !hp_dev || !out_dev || !grad_dev || !info_dev || N < 1 || N > GRID_BATCH_MAX_N || G < 1 ||
+      ld0 < N || !valid_stack(n_hidden, act, arch) || (kind != KIND_GAUSS && kind != KIND_STUDENT_T) ||
+      G > INT32_MAX)
+    return fail(SMNNGP_EINVAL, "smnngp_lml_grad_batch_f64: invalid argument");
+  GradBatchParams p{};
+  const size_t slot_bytes = carve_grad_slot(p, N, n_act_applications(n_hidden, arch));
+  const long long slots = workspace ? (long long)(workspace_bytes / slot_bytes) : 0;
+  if (slots < 1) return fail(SMNNGP_EWORKSPACE, "smnngp_lml_grad_batch_f64: workspace holds no slot");
+  p.K0dd = K0dd; p.q_d = q_d; p.y = y; p.hp = hp_dev; p.ld0 = ld0;
+  p.N = (int)N; p.G = (int)G; p.n_hidden = n_hidden; p.arch = arch; p.kind = kind;
+  p.ws = static_cast<char*>(workspace);
+  p.out = out_dev; p.grad = grad_dev; p.info = info_dev;
+  CU(launch_lml_grad_batch(s, p, act, slots));
+  return SMNNGP_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // host-buffer entry points
 // ---------------------------------------------------------------------------------------------------------

@@ -12,6 +12,7 @@
 // layer recursion in forward-mode dual arithmetic on the accumulators (3 values per entry) and contracts with the
 // G tile in registers.  Partial sums go to one slot per warp (fixed tile order per warp, fixed-order final
 // reduction): bit-reproducible.
+#include "closed_forms.cuh"
 #include "gemm_core.cuh"
 #include "kernels.cuh"
 #include "nngp_math.cuh"
@@ -20,26 +21,6 @@
 namespace smnngp {
 
 namespace {
-
-constexpr double kInv4Pi = 0.079577471545947667884;
-constexpr double kFourOverPi = 1.27323954473516268615;
-
-// ---- per-row dual tables ------------------------------------------------------------------------------------
-// tab3 = [3][n_act][tab_ld]:  plane 0: encoded marginal variance (relu: u, erf: 1/sqrt(1+2u))  (as qtable_kernel)
-//                             plane 1: f(u) du/dw_std,  plane 2: f(u) du/db_std
-// with f(u) = 1/(4 pi u) (relu: d phi / d u_i = s f(u_i)),  1/(1+2u) (erf: d phi / d u_i = -g x f(u_i))
-__device__ __forceinline__ void store_dual(double* tab3, long long plane, long long idx, double u, double duw,
-                                           double dub, int act) {
-  const double f = act == ACT_RELU ? (u > 0.0 ? kInv4Pi / u : 0.0) : 1.0 / (1.0 + 2.0 * u);
-  tab3[idx] = encode_var(u, act);
-  tab3[plane + idx] = f * duw;
-  tab3[2 * plane + idx] = f * dub;
-}
-// act_diag'(u)
-__device__ __forceinline__ double act_diag_deriv(double u, int act) {
-  if (act == ACT_RELU) return 0.5;
-  return kFourOverPi / ((1.0 + 2.0 * u) * sqrt(1.0 + 4.0 * u));
-}
 
 __global__ void qtable_dual_kernel(const double* __restrict__ X, long long ldx, int N, int D, int n_hidden, int act,
                                    int arch, const double* __restrict__ hp, double* __restrict__ tab3,
@@ -53,54 +34,7 @@ __global__ void qtable_dual_kernel(const double* __restrict__ X, long long ldx, 
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   if (lane != 0) return;
-  const double w = hp[HP_W], b = hp[HP_B];
-  const double w2 = w * w, b2 = b * b;
-  const long long plane = (long long)(n_act > 0 ? n_act : 1) * tab_ld;
-  double q = s / (double)D, dqw = 0.0, dqb = 0.0;
-  if (arch == ARCH_MLP) {
-    for (int a = 0; a < n_hidden; a++) {
-      const double u = w2 * q + b2, duw = 2.0 * w * q + w2 * dqw, dub = w2 * dqb + 2.0 * b;
-      store_dual(tab3, plane, a * tab_ld + row, u, duw, dub, act);
-      const double d = act_diag_deriv(u, act);
-      q = act_diag(u, act);
-      dqw = d * duw;
-      dqb = d * dub;
-    }
-  } else {
-    double u = w2 * q + b2, duw = 2.0 * w * q, dub = 2.0 * b;
-    for (int a = 0; a < n_hidden; a++) {
-      store_dual(tab3, plane, a * tab_ld + row, u, duw, dub, act);
-      const double ph = act_diag(u, act), d = act_diag_deriv(u, act);
-      u = u + (w2 * ph + b2);
-      const double nw = duw + (2.0 * w * ph + w2 * d * duw), nb = dub + (w2 * d * dub + 2.0 * b);
-      duw = nw;
-      dub = nb;
-    }
-    store_dual(tab3, plane, (long long)n_hidden * tab_ld + row, u, duw, dub, act);
-  }
-}
-
-// ---- dual layer step ------------------------------------------------------------------------------------------
-// in: k, dw, db (value and d/dw_std, d/db_std of the pre-activation cross-covariance), row / column table entries
-// out: phi and its duals
-template <int ACT>
-__device__ __forceinline__ void phi_dual(double k, double dw, double db, double e1, double e2, double fw, double fb,
-                                         double& ph, double& phw, double& phb) {
-  if (ACT == ACT_RELU) {
-    double s, a;
-    ph = phi_relu_parts(k, e1, e2, s, a);
-    const double pk = a * kInv2Pi;                 // (pi - theta) / (2 pi)
-    phw = fma(pk, dw, s * fw);                     // fw = f(u1) du1/dw + f(u2) du2/dw
-    phb = fma(pk, db, s * fb);
-  } else {
-    double x = 2.0 * k * e1 * e2;
-    x = fmin(fmax(x, -1.0), 1.0);
-    ph = kTwoOverPi * asin(x);
-    const double g = kTwoOverPi * rsqrt(fmax(1.0 - x * x, 1e-300));
-    const double pk = 2.0 * g * e1 * e2;
-    phw = fma(pk, dw, -g * x * fw);
-    phb = fma(pk, db, -g * x * fb);
-  }
+  fill_row_dual_tables(s, D, row, n_hidden, act, arch, hp, tab3, tab_ld, n_act);
 }
 
 struct GradParams {
@@ -181,22 +115,8 @@ __device__ __forceinline__ void grad_epilogue(const GradParams& p, double (&acc)
 #pragma unroll
           for (int e = 0; e < 2; e++) {
             const long long ci = a * tl + cc[ni][e];
-            const double e2 = t0[ci], fw = fw1 + t1[ci], fb = fb1 + t2[ci];
-            double kin = k[ni][e], dwin = dw[ni][e], dbin = db[ni][e];
-            if (!resnet) {                                         // Dense(512, W_std, b_std)
-              dwin = fma(w2, dwin, 2.0 * w * kin);
-              dbin = fma(w2, dbin, 2.0 * b);
-              kin = fma(w2, kin, b2);
-            }
-            double ph, phw, phb;
-            phi_dual<ACT>(kin, dwin, dbin, e1, e2, fw, fb, ph, phw, phb);
-            if (plain) {
-              k[ni][e] = ph; dw[ni][e] = phw; db[ni][e] = phb;
-            } else {                                               // ResBlock: z + Dense(act(z))
-              k[ni][e] = kin + fma(w2, ph, b2);
-              dw[ni][e] = dwin + fma(w2, phw, 2.0 * w * ph);
-              db[ni][e] = dbin + fma(w2, phb, 2.0 * b);
-            }
+            layer_step_dual<ACT>(k[ni][e], dw[ni][e], db[ni][e], e1, t0[ci], fw1 + t1[ci], fb1 + t2[ci], w, b, w2, b2,
+                                 resnet, plain);
           }
       }
       const double al_r = p.alpha[r];
@@ -284,16 +204,6 @@ cudaError_t launch_grad_fallback(cudaStream_t s, const GradParams& p) {
   return cudaGetLastError();
 }
 
-// digamma for x > 0: recurrence up to x >= 10, then the asymptotic series (error < 1e-17)
-__device__ double digamma_pos(double x) {
-  double r = 0.0;
-  while (x < 10.0) { r -= 1.0 / x; x += 1.0; }
-  const double f = 1.0 / (x * x);
-  const double t = f * (-1.0 / 12.0 + f * (1.0 / 120.0 + f * (-1.0 / 252.0 + f * (1.0 / 240.0 + f * (-1.0 / 132.0 +
-                   f * (691.0 / 32760.0 + f * (-1.0 / 12.0)))))));
-  return r + log(x) - 0.5 / x + t;
-}
-
 // one block: fixed-order sum of the slots, then the closed forms.  grad[6] = d loss / d hp, loss = -log p / N.
 __global__ void __launch_bounds__(1024) grad_finalize_kernel(const double* __restrict__ partial, long long slots,
                                                              const double* __restrict__ hp,
@@ -315,16 +225,7 @@ __global__ void __launch_bounds__(1024) grad_finalize_kernel(const double* __res
     __syncthreads();
   }
   if (threadIdx.x != 0) return;
-  const double n = (double)N, quad = *quad_p;
-  double dlp[6] = {red[0][0], red[1][0], red[2][0], red[3][0], 0.0, 0.0};
-  if (kind == KIND_STUDENT_T) {
-    const double a = hp[HP_ALPHA], b = hp[HP_BETA], t = a + 0.5 * n;
-    // quad / nu = quad / (2 b) does not depend on a; the N/2 log terms in a cancel
-    dlp[4] = -log1p(quad / (2.0 * b)) + digamma_pos(t) - digamma_pos(a);
-    dlp[5] = t * quad / (b * (2.0 * b + quad)) - 0.5 * n / b;
-  }
-  const bool bad = *info != 0;
-  for (int q = 0; q < 6; q++) grad[q] = bad ? __longlong_as_double(0x7ff8000000000000ll) : -dlp[q] / n;
+  grad_closed_form(red[0][0], red[1][0], red[2][0], red[3][0], hp, quad_p, kind, N, info, grad);
 }
 
 // alpha_i = sum_{k >= i} U[i,k] z[k]   (U = L^-T upper triangular, row-major): one block per row

@@ -152,6 +152,21 @@ struct GridBatchParams {
 // one persistent launch: min(slots, G) CTAs, each owns one slot and evaluates points blockIdx.x, + gridDim.x, ...
 cudaError_t launch_grid_batch(cudaStream_t s, const GridBatchParams& p, int act, long long slots);
 
+// ---- batched loss + gradient (grad_batch.cu) ----------------------------------------------------------------
+struct GradBatchParams {
+  const double *K0dd, *q_d, *y;                // cached base (smnngp_grid_base_f64, T = 0) and the targets
+  const double* hp;                            // [G][HP_COUNT]
+  long long ld0;
+  int N, G, n_hidden, arch, kind;
+  char* ws;                                    // slot k at ws + k * slot_bytes
+  long long slot_bytes, lda;                   // lda: row stride of a slot's (2N + 1)-row trapezoid
+  long long off_tab3, off_alpha;               // dual tables [3][n_act][N] and A^-1 y inside a slot (doubles)
+  double *out, *grad;                          // [G][4], [G][6]
+  int* info;                                   // [G]
+};
+// one persistent launch: min(slots, G) CTAs, each owns one slot and evaluates points blockIdx.x, + gridDim.x, ...
+cudaError_t launch_lml_grad_batch(cudaStream_t s, const GradBatchParams& p, int act, long long slots);
+
 // ---- gradient of the log marginal likelihood (grad.cu) -------------------------------------------------------
 // tab3 [3][n_act][tab_ld]: encoded marginal variances + the two dual planes the gradient epilogue needs
 cudaError_t launch_qtable_dual(cudaStream_t s, const double* X, long long ldx, int N, int D, int n_hidden, int act,

@@ -1,6 +1,6 @@
 // Device math of the NNGP layer recursion (experiments/nt_kernels.py:12-31, :83-103 with neural_tangents
 // semantics): diagonal maps, the branch-free ReLU arc-cosine step and the erf step, plus their partial
-// derivatives (used by the gradient pass, grad.cu).
+// derivatives (used by the gradient passes, grad.cu and grad_batch.cu).
 #pragma once
 #include "kernels.cuh"
 
@@ -139,6 +139,116 @@ __device__ __forceinline__ double layer_step(double k, double tr, double tc, dou
   if (!resnet) k = w2 * k + b2;
   const double ph = phi<ACT>(k, tr, tc);
   return plain ? ph : k + (w2 * ph + b2);
+}
+
+// K entry from its base value (X.X'^T / D): the recursion of gram_epilogue (gram.cu) on one element, then the final
+// Dense
+template <int ACT>
+__device__ __forceinline__ double nngp_entry(double k, const double* __restrict__ tab_r, long long ld_r, int r,
+                                             const double* __restrict__ tab_c, long long ld_c, int c, int n_act,
+                                             bool resnet, double w2, double b2, double v2) {
+  if (resnet) k = w2 * k + b2;
+  for (int a = 0; a < n_act; a++)
+    k = layer_step<ACT>(k, tab_r[a * ld_r + r], tab_c[a * ld_c + c], w2, b2, resnet, !resnet || a == n_act - 1);
+  return v2 * k;
+}
+
+// ---- forward-mode duals of the recursion (gradient w.r.t. w_std and b_std) -------------------------------------
+constexpr double kInv4Pi = 0.079577471545947667884;
+constexpr double kFourOverPi = 1.27323954473516268615;
+
+// per-row dual tables tab3 = [3][n_act][tab_ld]:
+//   plane 0: encoded marginal variance (relu: u, erf: 1/sqrt(1+2u))  (as fill_row_tables)
+//   plane 1: f(u) du/dw_std,  plane 2: f(u) du/db_std
+// with f(u) = 1/(4 pi u) (relu: d phi / d u_i = s f(u_i)),  1/(1+2u) (erf: d phi / d u_i = -g x f(u_i))
+__device__ __forceinline__ void store_dual(double* tab3, long long plane, long long idx, double u, double duw,
+                                           double dub, int act) {
+  const double f = act == ACT_RELU ? (u > 0.0 ? kInv4Pi / u : 0.0) : 1.0 / (1.0 + 2.0 * u);
+  tab3[idx] = encode_var(u, act);
+  tab3[plane + idx] = f * duw;
+  tab3[2 * plane + idx] = f * dub;
+}
+// act_diag'(u)
+__device__ __forceinline__ double act_diag_deriv(double u, int act) {
+  if (act == ACT_RELU) return 0.5;
+  return kFourOverPi / ((1.0 + 2.0 * u) * sqrt(1.0 + 4.0 * u));
+}
+
+// the dual tables of one row from its input variance q = ss / D (ss = ||x||^2; a cached q is passed with D = 1, exact)
+// n_act = n_act_applications(n_hidden, arch)
+__device__ __forceinline__ void fill_row_dual_tables(double ss, int D, int row, int n_hidden, int act, int arch,
+                                                     const double* __restrict__ hp, double* __restrict__ tab3,
+                                                     long long tab_ld, int n_act) {
+  const double w = hp[HP_W], b = hp[HP_B];
+  const double w2 = w * w, b2 = b * b;
+  const long long plane = (long long)(n_act > 0 ? n_act : 1) * tab_ld;
+  double q = ss / (double)D, dqw = 0.0, dqb = 0.0;
+  if (arch == ARCH_MLP) {
+    for (int a = 0; a < n_hidden; a++) {
+      const double u = w2 * q + b2, duw = 2.0 * w * q + w2 * dqw, dub = w2 * dqb + 2.0 * b;
+      store_dual(tab3, plane, a * tab_ld + row, u, duw, dub, act);
+      const double d = act_diag_deriv(u, act);
+      q = act_diag(u, act);
+      dqw = d * duw;
+      dqb = d * dub;
+    }
+  } else {
+    double u = w2 * q + b2, duw = 2.0 * w * q, dub = 2.0 * b;
+    for (int a = 0; a < n_hidden; a++) {
+      store_dual(tab3, plane, a * tab_ld + row, u, duw, dub, act);
+      const double ph = act_diag(u, act), d = act_diag_deriv(u, act);
+      u = u + (w2 * ph + b2);
+      const double nw = duw + (2.0 * w * ph + w2 * d * duw), nb = dub + (w2 * d * dub + 2.0 * b);
+      duw = nw;
+      dub = nb;
+    }
+    store_dual(tab3, plane, (long long)n_hidden * tab_ld + row, u, duw, dub, act);
+  }
+}
+
+// dual layer step.  in: k, dw, db (value and d/dw_std, d/db_std of the pre-activation cross-covariance), row / column
+// table entries; out: phi and its duals
+template <int ACT>
+__device__ __forceinline__ void phi_dual(double k, double dw, double db, double e1, double e2, double fw, double fb,
+                                         double& ph, double& phw, double& phb) {
+  if (ACT == ACT_RELU) {
+    double s, a;
+    ph = phi_relu_parts(k, e1, e2, s, a);
+    const double pk = a * kInv2Pi;                 // (pi - theta) / (2 pi)
+    phw = fma(pk, dw, s * fw);                     // fw = f(u1) du1/dw + f(u2) du2/dw
+    phb = fma(pk, db, s * fb);
+  } else {
+    double x = 2.0 * k * e1 * e2;
+    x = fmin(fmax(x, -1.0), 1.0);
+    ph = kTwoOverPi * asin(x);
+    const double g = kTwoOverPi * rsqrt(fmax(1.0 - x * x, 1e-300));
+    const double pk = 2.0 * g * e1 * e2;
+    phw = fma(pk, dw, -g * x * fw);
+    phb = fma(pk, db, -g * x * fb);
+  }
+}
+
+// One layer of the dual recursion on one entry (k, dw, db) in place: MLP layer, resnet block or trailing activation
+// (plain), as layer_step.  e1 / e2: plane 0 of the row / column; fw / fb: sums of the row's and column's planes 1 / 2.
+template <int ACT>
+__device__ __forceinline__ void layer_step_dual(double& k, double& dw, double& db, double e1, double e2, double fw,
+                                                double fb, double w, double b, double w2, double b2, bool resnet,
+                                                bool plain) {
+  double kin = k, dwin = dw, dbin = db;
+  if (!resnet) {                                         // Dense(512, W_std, b_std)
+    dwin = fma(w2, dwin, 2.0 * w * kin);
+    dbin = fma(w2, dbin, 2.0 * b);
+    kin = fma(w2, kin, b2);
+  }
+  double ph, phw, phb;
+  phi_dual<ACT>(kin, dwin, dbin, e1, e2, fw, fb, ph, phw, phb);
+  if (plain) {
+    k = ph; dw = phw; db = phb;
+  } else {                                               // ResBlock: z + Dense(act(z))
+    k = kin + fma(w2, ph, b2);
+    dw = dwin + fma(w2, phw, 2.0 * w * ph);
+    db = dbin + fma(w2, phb, 2.0 * b);
+  }
 }
 
 }  // namespace smnngp

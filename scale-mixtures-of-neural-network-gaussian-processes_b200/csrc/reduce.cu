@@ -3,13 +3,13 @@
 // variance (neural_tangents predict as used at spax/kernels.py:29-32; only diag(cov) is consumed downstream,
 // spax/likelihoods.py:31,62) and the per-test-point log density (spax/likelihoods.py:52-65, :30-33).
 // All reductions run in a fixed order (deterministic).
+#include "closed_forms.cuh"
 #include "kernels.cuh"
 
 namespace smnngp {
 
 namespace {
 
-constexpr double kPi = 3.14159265358979323846;
 __device__ __forceinline__ double qnan() { return __longlong_as_double(0x7ff8000000000000ll); }
 
 __global__ void sumsq_kernel(const double* __restrict__ z, long long n, double* __restrict__ out) {
@@ -27,24 +27,7 @@ __global__ void sumsq_kernel(const double* __restrict__ z, long long n, double* 
 
 __global__ void lml_finalize_kernel(const double* __restrict__ scal, const double* __restrict__ hp, int kind,
                                     long long N, const int* __restrict__ info, double* __restrict__ out) {
-  const double logdet = scal[SC_LOGDET], zz = scal[SC_QUAD];
-  const double n = (double)N;
-  double lml;
-  if (kind == KIND_STUDENT_T) {
-    // Sigma = (b/a)(K + eps I): chol(c S) = sqrt(c) chol(S)  =>  log-det += N/2 log c, quadratic form /= c
-    const double a = hp[HP_ALPHA], b = hp[HP_BETA];
-    const double c = b / a, df = 2.0 * a, t = 0.5 * (df + n);
-    const double half_logdet = logdet + 0.5 * n * log(c);
-    const double quad = zz / c;
-    lml = -t * log(1.0 + quad / df) - 0.5 * n * log(df * kPi) + lgamma(t) - lgamma(0.5 * df) - half_logdet;
-  } else {
-    lml = -0.5 * zz - 0.5 * n * log(2.0 * kPi) - logdet;
-  }
-  if (*info != 0) lml = qnan();
-  out[0] = lml;
-  out[1] = -lml / n;
-  out[2] = logdet;
-  out[3] = zz;
+  lml_closed_form(scal[SC_LOGDET], scal[SC_QUAD], hp, kind, N, info, out);
 }
 
 constexpr int PRED_MAXC = 16;

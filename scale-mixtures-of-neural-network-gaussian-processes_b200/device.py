@@ -503,6 +503,71 @@ class GridSearch:
         return sweep_eps(eps_list, evaluate, t=self.t, device=self.y.device, group=group)
 
 
+def _grad_batch_wins(n, g):
+    """Whether ``LossGradBatch.points`` evaluates G points of N training rows in one batched launch rather than one
+    ``lml_grad`` call after the other.  Provisional: the form of ``_batch_wins`` (a CTA-point costs ~(N / 404)^1.6
+    per-call evaluations), with a lower constant because one ``lml_grad`` call is ~2x a ``grid_point`` call at N = 404.
+    ``profiles/grad_batch_bench.py`` times both paths at N = 404 .. 4096 and G = 1 .. 1100 to re-derive it."""
+    return n <= GRID_BATCH_MAX_N and g >= 2.0 * (n / 404.0) ** 1.6
+
+
+class LossGradBatch:
+    """``SPR.loss`` and its six-scalar gradient at many hyper-parameter points over the same data - multi-start
+    training, or gradient refinement of the best points of a grid search.  X.X^T / D and the input variances are cached
+    once (smnngp_grid_base_f64 with no test rows); ``points(hps, kind)`` evaluates every row of ``hps``."""
+
+    def __init__(self, x, y, *, spec: StackSpec):
+        _require_cuda()
+        self.lib = _lib.load()
+        self.spec = spec
+        self.x = _f64(x)
+        self.y = _f64(y, self.x.device)
+        self.n, d = self.x.shape
+        dev = self.x.device
+        self.ld0 = (self.n + 15) // 16 * 16
+        self.k0dd = torch.empty((self.n, self.ld0), dtype=torch.float64, device=dev)
+        self.q_d = torch.empty(self.n, dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            rc = self.lib.smnngp_grid_base_f64(_stream(dev), _p(self.x), None, self.n, 0, d, _p(self.k0dd), self.ld0,
+                                               None, 0, _p(self.q_d), None)
+        _lib.check(rc, "grid_base")
+
+    def points(self, hps, kind="student_t"):
+        """(out [G, 4], grad [G, 6], info [G]) for the rows of ``hps`` [G, 6] (device operand rows, see make_hp): row g
+        is what ``lml_grad(x, y, hp=hps[g], kind=kind)`` returns, up to rounding.  Where one launch for every point is
+        faster (``_grad_batch_wins``) a CTA evaluates each point in its own workspace slot (smnngp_lml_grad_batch_f64);
+        elsewhere, and always for N > 4096, the points run one ``lml_grad`` call after the other."""
+        dev = self.x.device
+        hps = _f64(hps, dev)
+        if hps.ndim != 2 or hps.shape[1] != 6:
+            raise ValueError("hps must be [G, 6]")
+        if kind not in KIND:
+            raise ValueError(f"unknown likelihood kind '{kind}'")
+        g = hps.shape[0]
+        if not _grad_batch_wins(self.n, g):
+            rows = [lml_grad(self.x, self.y, spec=self.spec, hp=hps[i], kind=kind) for i in range(g)]
+            return (torch.stack([r[0] for r in rows]), torch.stack([r[1] for r in rows]),
+                    torch.cat([r[2] for r in rows]))
+        nh, act, arch = self.spec.ids()
+        out = torch.empty((g, 4), dtype=torch.float64, device=dev)
+        grad = torch.empty((g, 6), dtype=torch.float64, device=dev)
+        info = torch.empty(g, dtype=torch.int32, device=dev)
+        # every slot a CTA the device keeps resident (lml_grad_batch_kernel: two per SM), as far as half the free
+        # memory holds them (a slot is ~268 MB at N = 4096); more slots would only wait
+        one = self.lib.smnngp_lml_grad_batch_workspace_bytes(self.n, nh, arch, 1)
+        with torch.cuda.device(dev):
+            free = torch.cuda.mem_get_info(dev)[0]
+        slots = max(1, min(g, 2 * torch.cuda.get_device_properties(dev).multi_processor_count, free // 2 // one))
+        ws_bytes = slots * one
+        with torch.cuda.device(dev):
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            rc = self.lib.smnngp_lml_grad_batch_f64(_stream(dev), _p(self.k0dd), self.ld0, _p(self.q_d), _p(self.y),
+                                                    self.n, g, nh, act, arch, _p(hps), KIND[kind], _p(ws), ws_bytes,
+                                                    _p(out), _p(grad), _p(info))
+        _lib.check(rc, "lml_grad_batch")
+        return out, grad, info
+
+
 def set_panel_width(nb: int):
     _lib.load().smnngp_set_panel_width(int(nb))
 

@@ -11,7 +11,7 @@ from .utils import jitter
 from .. import device as _dev
 from ..nt_kernels import KernelFn
 
-__all__ = ["SPR", "DistributedSPR"]
+__all__ = ["SPR", "DistributedSPR", "MultiStartSPR"]
 
 
 class SPR(Module):
@@ -153,3 +153,66 @@ class DistributedSPR(SPR):
             if s is not None and hasattr(s, "close"):
                 s.close()
         self._grad_solver, self._predict_solvers = None, {}
+
+
+def _softplus(x):
+    return torch.logaddexp(x, torch.zeros_like(x))                                    # bijectors.Softplus on a tensor
+
+
+def _softplus_inverse(x):
+    return torch.where(x < 20.0, torch.log(torch.expm1(torch.clamp(x, max=20.0))), x)
+
+
+class MultiStartSPR:
+    """R copies of an SPR over the same data, trained together: multi-start restarts of the six non-convex scalars.
+    ``starts`` [R, 6] holds the safe values {w_std, b_std, last_w_std, eps, alpha, beta} of every restart; the stack
+    comes from ``kernel.get_kernel_fn()`` and the kind from the likelihood (their own variables are not used).  The
+    unconstrained variables are one device tensor ``raw`` [R, 6] (softplus, spax/bijectors.py), stepped by
+    ``BatchAdam``.  Under a Gaussian likelihood alpha and beta are not variables (``mask`` is False there): their
+    gradient is 0 and they are never updated."""
+
+    def __init__(self, kernel, likelihood, x_data, y_data, y_mean, y_std, *, starts):
+        kernel_fn = kernel.get_kernel_fn()
+        if not (isinstance(kernel_fn, KernelFn) and getattr(likelihood, "kind", None) in _dev.KIND):
+            raise TypeError("MultiStartSPR needs a kernel_fn built by smnngp nt_kernels and a spax likelihood")
+        self.spec, self.kind = kernel_fn.spec, likelihood.kind
+        if isinstance(x_data, torch.Tensor):
+            dev = x_data.device
+        else:
+            dev = torch.device("cuda" if torch.cuda.is_available() else "cpu")
+        to_dev = lambda a: a.to(dev, torch.float64) if isinstance(a, torch.Tensor) else torch.as_tensor(
+            np.ascontiguousarray(a, dtype=np.float64), device=dev)
+        self.x_data, self.y_data = to_dev(x_data), to_dev(y_data)
+        self.y_mean, self.y_std = float(y_mean), float(y_std)
+        self.num_data = self.x_data.shape[0]
+        starts = to_dev(starts)
+        if starts.ndim != 2 or starts.shape[1] != 6:
+            raise ValueError("starts must be [R, 6]")
+        self.raw = _softplus_inverse(starts).contiguous()
+        self.mask = torch.ones(6, dtype=torch.bool, device=dev)
+        if self.kind != "student_t":
+            self.mask[4:] = False
+        self._batch = None
+
+    def safe_values(self):
+        """[R, 6] constrained values {w_std, b_std, last_w_std, eps, alpha, beta}."""
+        return _softplus(self.raw)
+
+    def loss_and_grad(self):
+        """(loss [R], grad_raw [R, 6], info [R]) in one ``LossGradBatch.points`` call: loss = SPR.loss of every
+        restart, grad_raw = d loss / d raw (the softplus chain rule applied on the device, zero where ``mask`` is
+        False)."""
+        if self._batch is None:
+            self._batch = _dev.LossGradBatch(self.x_data, self.y_data, spec=self.spec)
+        out, grad, info = self._batch.points(self.safe_values(), self.kind)
+        g = torch.where(self.mask, grad * torch.sigmoid(self.raw), torch.zeros_like(grad))
+        return out[:, 1], g, info
+
+    def test_nll(self, x, y):
+        """[R] SPR.test_nll of every restart (one fused call per restart)."""
+        x = torch.as_tensor(x, dtype=torch.float64, device=self.x_data.device)
+        y = torch.as_tensor(y, dtype=torch.float64, device=self.x_data.device)
+        hps = self.safe_values()
+        rows = [_dev.test_nll(self.x_data, self.y_data, x, y, self.y_mean, self.y_std, spec=self.spec, hp=hps[r],
+                              kind=self.kind)[0] for r in range(hps.shape[0])]
+        return torch.stack(rows)

@@ -5,7 +5,7 @@ import math
 
 import numpy as np
 
-__all__ = ["Adam"]
+__all__ = ["Adam", "BatchAdam"]
 
 
 class Adam:
@@ -38,3 +38,36 @@ class Adam:
             self.m[k] = self.beta1 * self.m[k] + (1.0 - self.beta1) * g
             self.v[k] = self.beta2 * self.v[k] + (1.0 - self.beta2) * g * g
             var.assign(var.value - lr_t * self.m[k] / np.sqrt(self.v[k] + self.eps))
+
+
+class BatchAdam:
+    """``Adam`` on R models at once: the unconstrained variables of every restart are one [R, 6] tensor (``raw``, updated
+    in place on its device), and one step applies objax's update elementwise, ``p -= lr_t * m * rsqrt(v + eps)`` with eps
+    inside the square root, exactly like ``Adam``.  Rows never mix: a NaN gradient poisons only its own row.
+    mask: [6] (or [R, 6]) booleans, False for entries that are not variables (Gaussian likelihood: alpha, beta); those
+    are never updated."""
+
+    def __init__(self, raw, mask=None, beta1: float = 0.9, beta2: float = 0.999, eps: float = 1e-8):
+        import torch
+        self.raw = raw
+        self.mask = None if mask is None else torch.as_tensor(mask, dtype=torch.bool, device=raw.device)
+        self.beta1, self.beta2, self.eps = beta1, beta2, eps
+        self.step = 0
+        self.m = torch.zeros_like(raw)
+        self.v = torch.zeros_like(raw)
+
+    def __call__(self, lr: float, grad, active=None):
+        """grad: [R, 6] d loss / d raw (what ``MultiStartSPR.loss_and_grad`` returns).  active: optional [R] booleans;
+        rows that are False (frozen restarts) keep their variables."""
+        import torch
+        self.step += 1
+        lr_t = lr * math.sqrt(1.0 - self.beta2 ** self.step) / (1.0 - self.beta1 ** self.step)
+        self.m = self.beta1 * self.m + (1.0 - self.beta1) * grad
+        self.v = self.beta2 * self.v + (1.0 - self.beta2) * grad * grad
+        new = self.raw - lr_t * self.m / torch.sqrt(self.v + self.eps)
+        keep = torch.zeros_like(self.raw, dtype=torch.bool)
+        if self.mask is not None:
+            keep |= ~self.mask
+        if active is not None:
+            keep |= ~torch.as_tensor(active, dtype=torch.bool, device=self.raw.device)[:, None]
+        self.raw.copy_(torch.where(keep, self.raw, new))
