@@ -168,6 +168,28 @@ int smnngp_lml_grad_batch_f64(void* stream, const double* K0dd, int64_t ld0, con
                               int64_t N, int64_t G, int n_hidden, int act, int arch, const double* hp_dev, int kind,
                               void* workspace, size_t workspace_bytes, double* out_dev, double* grad_dev,
                               int* info_dev);
+/* test_nll_batch  SPR.test_nll at G points in ONE launch for N <= 4096 (the validation / test NLL of multi-start
+ *             training, selection of grid points by held-out NLL).  K0dd / K0td / q_d / q_t are the bases of grid_base,
+ *             y [N] the training targets, yt [T] the standardised test targets; hp_dev [G][6]; kind, y_mean and
+ *             y_std as smnngp_test_nll_f64.  nll_out [G] and info_dev [G]; mean_out, var_out and logp_out are [G][T]
+ *             each and may be NULL.  Row g is what smnngp_test_nll_f64 returns for hp_dev + 6 g, up to rounding (same
+ *             matrices, different blocking).  mean / var of a point are NaN when its predictive factorisation
+ *             (K + eps tr(K)/N I) fails; nll and logp are NaN when it or the Student-t one (K + 1e-6 (alpha/beta) I)
+ *             fails; info_dev[g] is the first bad pivot (1-based) of the predictive factorisation, else of the
+ *             Student-t one, else 0.  No point affects another, and nll does not depend on which optional outputs
+ *             are asked for: a point's outputs are the same bits in any batch, order or slot count.  The slot count
+ *             is workspace_bytes / smnngp_test_nll_batch_workspace_bytes(.., 1); each slot holds the (N + T + 1) x N
+ *             trapezoid, the layer tables and 2T doubles of mean / var.  Fewer than one slot: SMNNGP_EWORKSPACE;
+ *             N < 1, N > 4096, T < 1, G < 1, a null required pointer, ld0 or ld0t < N, an invalid stack or kind:
+ *             SMNNGP_EINVAL, both before anything is enqueued.  Enqueue-only (one kernel launch), no allocation,
+ *             graph-capturable. */
+size_t smnngp_test_nll_batch_workspace_bytes(int64_t N, int64_t T, int n_hidden, int arch, int64_t slots);
+int smnngp_test_nll_batch_f64(void* stream, const double* K0dd, int64_t ld0, const double* K0td, int64_t ld0t,
+                              const double* q_d, const double* q_t, const double* y, const double* yt,
+                              int64_t N, int64_t T, int64_t G, int n_hidden, int act, int arch,
+                              const double* hp_dev, int kind, double y_mean, double y_std,
+                              void* workspace, size_t workspace_bytes,
+                              double* nll_out, double* mean_out, double* var_out, double* logp_out, int* info_dev);
 
 /* ---- posterior draw stage of the classification / ensemble configuration (SURVEY section 8f, row N2).
  * mean [T, C]; var [T] (shared by the classes, var_per_class = 0) or [C, T] (var_per_class = 1); kind STUDENT_T:

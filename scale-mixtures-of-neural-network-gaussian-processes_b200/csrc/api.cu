@@ -709,6 +709,58 @@ int smnngp_lml_grad_batch_f64(void* stream, const double* K0dd, int64_t ld0, con
   return SMNNGP_OK;
 }
 
+// SPR.test_nll at every point in one launch (test_nll_batch.cu): the trapezoid, the tables, then the mean / var scratch
+namespace {
+size_t carve_test_nll_slot(TestNllBatchParams& p, long long N, long long T, int n_act) {
+  const size_t na = (size_t)(n_act > 0 ? n_act : 1);
+  Carver c(nullptr);
+  p.lda = round_up(N, 16);
+  c.take<double>((size_t)(N + T + 1) * p.lda);
+  p.off_tab = (long long)(c.total() / 8);
+  c.take<double>(na * N);
+  p.off_q = (long long)(c.total() / 8);
+  c.take<double>(N);
+  p.off_tab_t = (long long)(c.total() / 8);
+  c.take<double>(na * T);
+  p.off_q_t = (long long)(c.total() / 8);
+  c.take<double>(T);
+  p.off_mv = (long long)(c.total() / 8);
+  c.take<double>(2 * (size_t)T);
+  p.slot_bytes = (long long)c.total();
+  return c.total();
+}
+}  // namespace
+
+size_t smnngp_test_nll_batch_workspace_bytes(int64_t N, int64_t T, int n_hidden, int arch, int64_t slots) {
+  TestNllBatchParams p{};
+  return (size_t)(slots > 0 ? slots : 0) * carve_test_nll_slot(p, N, T, n_act_applications(n_hidden, arch));
+}
+
+int smnngp_test_nll_batch_f64(void* stream, const double* K0dd, int64_t ld0, const double* K0td, int64_t ld0t,
+                              const double* q_d, const double* q_t, const double* y, const double* yt, int64_t N,
+                              int64_t T, int64_t G, int n_hidden, int act, int arch, const double* hp_dev, int kind,
+                              double y_mean, double y_std, void* workspace, size_t workspace_bytes, double* nll_out,
+                              double* mean_out, double* var_out, double* logp_out, int* info_dev) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  if (!K0dd || !K0td || !q_d || !q_t || !y || !yt || !hp_dev || !nll_out || !info_dev || N < 1 ||
+      N > GRID_BATCH_MAX_N || T < 1 || G < 1 || ld0 < N || ld0t < N || !valid_stack(n_hidden, act, arch) ||
+      (kind != KIND_GAUSS && kind != KIND_STUDENT_T) || N + T + 1 > INT32_MAX || G > INT32_MAX)
+    return fail(SMNNGP_EINVAL, "smnngp_test_nll_batch_f64: invalid argument");
+  TestNllBatchParams p{};
+  const size_t slot_bytes = carve_test_nll_slot(p, N, T, n_act_applications(n_hidden, arch));
+  const long long slots = workspace ? (long long)(workspace_bytes / slot_bytes) : 0;
+  if (slots < 1) return fail(SMNNGP_EWORKSPACE, "smnngp_test_nll_batch_f64: workspace holds no slot");
+  p.K0dd = K0dd; p.K0td = K0td; p.q_d = q_d; p.q_t = q_t; p.y = y; p.yt = yt; p.hp = hp_dev;
+  p.ld0 = ld0; p.ld0t = ld0t;
+  p.N = (int)N; p.T = (int)T; p.G = (int)G; p.n_hidden = n_hidden; p.arch = arch; p.kind = kind;
+  p.y_mean = y_mean; p.y_std = y_std;
+  p.ws = static_cast<char*>(workspace);
+  p.nll = nll_out; p.mean = mean_out; p.var = var_out; p.logp = logp_out; p.info = info_dev;
+  CU(launch_test_nll_batch(s, p, act, slots));
+  return SMNNGP_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // host-buffer entry points
 // ---------------------------------------------------------------------------------------------------------

@@ -1,5 +1,5 @@
-// Scalar closed forms of SPR.loss and of its gradient, shared by the per-call finalize kernels (reduce.cu, grad.cu)
-// and the batched loss + gradient (grad_batch.cu).
+// Scalar closed forms of SPR.loss, of its gradient and of the log density of SPR.test_nll, shared by the per-call
+// finalize kernels (reduce.cu, grad.cu) and the batched kernels (grad_batch.cu, test_nll_batch.cu).
 #pragma once
 #include "nngp_math.cuh"
 
@@ -26,6 +26,34 @@ __device__ __forceinline__ void lml_closed_form(double logdet, double zz, const 
   out[1] = -lml / n;
   out[2] = logdet;
   out[3] = zz;
+}
+
+// jax.scipy.stats.t.logpdf (spax/likelihoods.py:64)
+__device__ __forceinline__ double t_logpdf(double x, double df, double loc, double scale) {
+  const double z = (x - loc) / scale;
+  const double norm = lgamma(0.5 * df) + 0.5 * log(df) + 0.5 * log(scale * scale * kPi) - lgamma(0.5 * (df + 1.0));
+  return -(norm + 0.5 * (df + 1.0) * log1p(z * z / df));
+}
+
+// log density of one de-standardised test target x under the predictive of SPR.test_nll with mean m and variance cv
+// (spax/likelihoods.py:52-65 Student-t, :30-33 Gaussian); *quad2 = ||L2^-1 y||^2 with L2 = chol(K + 1e-6 (a/b) I) is
+// read under Student-t only
+__device__ __forceinline__ double test_logpdf(double x, double m, double cv, const double* __restrict__ hp, int kind,
+                                              long long N, const double* __restrict__ quad2) {
+  double lp;
+  if (kind == KIND_STUDENT_T) {
+    const double a = hp[HP_ALPHA], b = hp[HP_BETA];
+    const double df = 2.0 * a, cond_df = df + (double)N;
+    // y^T ((b/a) K + 1e-6 I)^-1 y = (a/b) ||L2^-1 y||^2
+    const double d = df + (a / b) * (*quad2);
+    const double sigma = sqrt(d / cond_df * b / a * cv);
+    lp = t_logpdf(x, cond_df, m, sigma);
+  } else {
+    const double sigma = sqrt(cv);
+    const double z = (x - m) / sigma;
+    lp = -0.5 * log(2.0 * kPi) - log(sigma) - 0.5 * z * z;
+  }
+  return lp;
 }
 
 namespace {

@@ -167,6 +167,24 @@ struct GradBatchParams {
 // one persistent launch: min(slots, G) CTAs, each owns one slot and evaluates points blockIdx.x, + gridDim.x, ...
 cudaError_t launch_lml_grad_batch(cudaStream_t s, const GradBatchParams& p, int act, long long slots);
 
+// ---- batched test NLL (test_nll_batch.cu) --------------------------------------------------------------------
+struct TestNllBatchParams {
+  const double *K0dd, *K0td, *q_d, *q_t, *y;   // cached bases (smnngp_grid_base_f64) and the targets
+  const double* yt;                            // [T] standardised test targets
+  const double* hp;                            // [G][HP_COUNT]
+  long long ld0, ld0t;
+  int N, T, G, n_hidden, arch, kind;
+  double y_mean, y_std;
+  char* ws;                                    // slot k at ws + k * slot_bytes
+  long long slot_bytes, lda;                   // lda: row stride of a slot's (N + T + 1)-row trapezoid
+  long long off_tab, off_q, off_tab_t, off_q_t, off_mv;   // layer tables, [2][T] mean / var inside a slot (doubles)
+  double* nll;                                 // [G]
+  double *mean, *var, *logp;                   // [G][T] each, may be null
+  int* info;                                   // [G]
+};
+// one persistent launch: min(slots, G) CTAs, each owns one slot and evaluates points blockIdx.x, + gridDim.x, ...
+cudaError_t launch_test_nll_batch(cudaStream_t s, const TestNllBatchParams& p, int act, long long slots);
+
 // ---- gradient of the log marginal likelihood (grad.cu) -------------------------------------------------------
 // tab3 [3][n_act][tab_ld]: encoded marginal variances + the two dual planes the gradient epilogue needs
 cudaError_t launch_qtable_dual(cudaStream_t s, const double* X, long long ldx, int N, int D, int n_hidden, int act,

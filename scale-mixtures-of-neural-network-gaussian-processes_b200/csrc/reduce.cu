@@ -66,12 +66,6 @@ __global__ void __launch_bounds__(256) predict_finalize_kernel(const double* __r
   }
 }
 
-__device__ __forceinline__ double t_logpdf(double x, double df, double loc, double scale) {
-  const double z = (x - loc) / scale;
-  const double norm = lgamma(0.5 * df) + 0.5 * log(df) + 0.5 * log(scale * scale * kPi) - lgamma(0.5 * (df + 1.0));
-  return -(norm + 0.5 * (df + 1.0) * log1p(z * z / df));
-}
-
 __global__ void __launch_bounds__(1024) test_nll_finalize_kernel(
     const double* __restrict__ mean, const double* __restrict__ var, const double* __restrict__ ytest, int T,
     long long N, double y_mean, double y_std, const double* __restrict__ hp, int kind,
@@ -84,19 +78,7 @@ __global__ void __launch_bounds__(1024) test_nll_finalize_kernel(
     const double x = ytest[t] * y_std + y_mean;
     const double m = mean[t] * y_std + y_mean;
     const double cv = var[t] * (y_std * y_std);
-    double lp;
-    if (kind == KIND_STUDENT_T) {
-      const double a = hp[HP_ALPHA], b = hp[HP_BETA];
-      const double df = 2.0 * a, cond_df = df + (double)N;
-      // y^T ((b/a) K + 1e-6 I)^-1 y = (a/b) ||L2^-1 y||^2 with L2 = chol(K + 1e-6 (a/b) I)
-      const double d = df + (a / b) * (*quad2);
-      const double sigma = sqrt(d / cond_df * b / a * cv);
-      lp = t_logpdf(x, cond_df, m, sigma);
-    } else {
-      const double sigma = sqrt(cv);
-      const double z = (x - m) / sigma;
-      lp = -0.5 * log(2.0 * kPi) - log(sigma) - 0.5 * z * z;
-    }
+    double lp = test_logpdf(x, m, cv, hp, kind, N, quad2);
     if (bad) lp = qnan();
     if (logp) logp[t] = lp;
     acc += lp;

@@ -1,6 +1,6 @@
-// In-CTA building blocks of the batched kernels (grid_batch.cu, grad_batch.cu): one CTA of GB_THREADS threads owns a
-// workspace slot and works on one point at a time - the Gram rebuilt from its cached base, and a blocked Cholesky of
-// the slot.
+// In-CTA building blocks of the batched kernels (grid_batch.cu, grad_batch.cu, test_nll_batch.cu): one CTA of
+// GB_THREADS threads owns a workspace slot and works on one point at a time - the Gram rebuilt from its cached base, a
+// blocked Cholesky of the slot, and the predictive of a point.
 //
 // Cholesky of a slot (A row-major, lda, rows 0..N-1 lower = the matrix, rows N..M-1 carried), 64-column outer panels:
 //   per 16 columns:  the 16 x 16 diagonal block is staged to shared memory and factored + inverted by one warp
@@ -48,6 +48,22 @@ __device__ void build_gram(const P& p, const double* __restrict__ hp, const doub
 
 __device__ void copy_row(const double* __restrict__ src, double* __restrict__ dst, int n) {
   for (int i = threadIdx.x; i < n; i += GB_THREADS) dst[i] = src[i];
+}
+
+// rows N..N+T-1 of the slot = K_td
+template <int ACT, class P>
+__device__ void build_cross(const P& p, const double* __restrict__ hp, const double* __restrict__ tab,
+                            const double* __restrict__ tab_t, double* __restrict__ A) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const bool resnet = p.arch == ARCH_RESNET;
+  const int n_act = n_act_applications(p.n_hidden, p.arch);
+  const double w2 = hp[HP_W] * hp[HP_W], b2 = hp[HP_B] * hp[HP_B], v2 = hp[HP_V] * hp[HP_V];
+  for (int t = warp; t < p.T; t += GB_WARPS) {
+    const double* src = p.K0td + (long long)t * p.ld0t;
+    double* dst = A + (long long)(p.N + t) * p.lda;
+    for (int c = lane; c < p.N; c += 32)
+      dst[c] = nngp_entry<ACT>(src[c], tab_t, p.T, t, tab, p.N, c, n_act, resnet, w2, b2, v2);
+  }
 }
 
 // 8-row strip r0.. of the 16 columns at j0 (w valid) <- strip * inv(L_jj)^T, in place (rows < M)
@@ -272,6 +288,58 @@ __device__ void syrk_upper_slot(const double* __restrict__ U, long long ldu, int
       }
     }
   }
+}
+
+// The predictive of one point with the relative regulariser (what smnngp_grid_point_f64 and the first half of
+// smnngp_test_nll_f64 compute), for the point's scalars hp:
+//   1. layer tables of the train rows (tab, q) and the test rows (tab_t, q_t), tr(K)/N by a fixed-order block sum;
+//   2. the trapezoid K + eps tr(K)/N I (lower) | K_td | y^T in the slot A, factor_slot - the carried rows come out as
+//      v_t = K_td L^-T and z = (L^-1 y)^T - then, per test row t, lane 0 of one warp calls
+//      emit(t, ||v_t||^2, v_t . z, bad) with bad = the factorisation's *bad_s: mean_t = v_t . z and
+//      var_t = q_t[t] - ||v_t||^2 (emit forms var_t itself, so that it reads q_t only for a good point).
+// tid, lane, warp, N and T are the caller's; eps is set to hp[HP_EPS].  Returns bad; ends on a __syncthreads (the
+// slot is free again, emit's stores are visible to the CTA).
+template <int ACT, class P, class Emit>
+__device__ __forceinline__ int predictive_slot(const P& p, const double* __restrict__ hp, double* __restrict__ A,
+                                               double* __restrict__ tab, double* __restrict__ q,
+                                               double* __restrict__ tab_t, double* __restrict__ q_t,
+                                               double* __restrict__ smem, double* __restrict__ red, int* bad_s,
+                                               int tid, int lane, int warp, int N, int T, double& eps, Emit&& emit) {
+  double qs = 0.0;
+  for (int r = tid; r < N; r += GB_THREADS) {
+    fill_row_tables(p.q_d[r], r, p.n_hidden, ACT, p.arch, hp, tab, N, q);
+    qs += q[r];
+  }
+  for (int t = tid; t < T; t += GB_THREADS) fill_row_tables(p.q_t[t], t, p.n_hidden, ACT, p.arch, hp, tab_t, T, q_t);
+  const double trmean = block_sum<GB_THREADS>(qs, red) / (double)N;   // its __syncthreads also publishes the tables
+  eps = hp[HP_EPS];
+
+  build_gram<ACT>(p, hp, tab, A, eps * trmean);
+  build_cross<ACT>(p, hp, tab, tab_t, A);
+  copy_row(p.y, A + (long long)(N + T) * p.lda, N);
+  __syncthreads();
+  double lsum = 0.0;
+  factor_slot<false>(A, p.lda, N + T + 1, N, smem, bad_s, lsum);
+  __syncthreads();
+  const int bad = *bad_s;
+  const double* z = A + (long long)(N + T) * p.lda;
+  for (int t = warp; t < T; t += GB_WARPS) {
+    const double* v = A + (long long)(N + t) * p.lda;
+    double vv = 0.0, vz = 0.0;
+    for (int n = lane; n < N; n += 32) {
+      const double x = v[n];
+      vv = fma(x, x, vv);
+      vz = fma(x, z[n], vz);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      vv += __shfl_xor_sync(0xffffffffu, vv, o);
+      vz += __shfl_xor_sync(0xffffffffu, vz, o);
+    }
+    if (lane == 0) emit(t, vv, vz, bad);
+  }
+  __syncthreads();
+  return bad;
 }
 
 }  // namespace

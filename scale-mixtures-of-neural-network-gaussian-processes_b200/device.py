@@ -414,7 +414,9 @@ def _batch_wins(n, g):
     point after the other.  Up to the resident slots the batch costs what one CTA needs for one point; that is
     3.2, 8.9, 38 and 130 times a ``point`` call at N = 404, 824, 2048 and 4096 (profiles/r03_grid_batch.jsonl, B200 at
     1000 W), ~3.2 (N / 404)^1.6.  Past the slots the batch runs in waves of at least 148 points, which still beats the
-    loop wherever one wave does."""
+    loop wherever one wave does.  ``GridSearch.test_nll`` uses the same rule: a batched test-NLL point costs about a
+    batched grid point (the same two factorisations) and a ``test_nll`` call about a ``point`` call
+    (profiles/nll_batch_bench.py times both paths)."""
     return n <= GRID_BATCH_MAX_N and g >= 3.2 * (n / 404.0) ** 1.6
 
 
@@ -430,6 +432,7 @@ class GridSearch:
         x = _f64(x)
         self.y = _f64(y, x.device)
         xt = _f64(x_test, x.device)
+        self.x, self.x_test = x, xt                  # for the per-point test_nll loop
         self.n, d = x.shape
         self.t = xt.shape[0]
         dev = x.device
@@ -488,6 +491,49 @@ class GridSearch:
                                                 arch, _p(hps), _p(ws), ws_bytes, _p(mean), _p(var), _p(out), _p(info))
         _lib.check(rc, "grid_batch")
         return mean, var, 2.0 * out[:, 0], out[:, 1], info
+
+    def test_nll(self, hps, y_test, y_mean, y_std, kind="student_t"):
+        """``SPR.test_nll`` on the test rows at every row of ``hps`` [G, 6] (device operand rows, see make_hp):
+        (nll [G], mean [G, T], var [G, T], info [G]), row g what ``test_nll(x, y, x_test, y_test, y_mean, y_std,
+        hp=hps[g], kind=kind)`` returns, up to rounding.  ``y_test`` [T] holds the standardised test targets.  Where
+        one launch for every point is faster (``_batch_wins``) a CTA evaluates each point in its own workspace slot
+        (smnngp_test_nll_batch_f64); elsewhere, and always for N > 4096, the points run one ``test_nll`` call after
+        the other."""
+        dev = self.y.device
+        hps = _f64(hps, dev)
+        if hps.ndim != 2 or hps.shape[1] != 6:
+            raise ValueError("hps must be [G, 6]")
+        if kind not in KIND:
+            raise ValueError(f"unknown likelihood kind '{kind}'")
+        yt = _f64(y_test, dev)
+        if tuple(yt.shape) != (self.t,):
+            raise ValueError(f"y_test must be [{self.t}]")
+        g = hps.shape[0]
+        if not _batch_wins(self.n, g):
+            rows = [test_nll(self.x, self.y, self.x_test, yt, y_mean, y_std, spec=self.spec, hp=hps[i], kind=kind)
+                    for i in range(g)]
+            return tuple(torch.stack([r[k] for r in rows]) for k in range(3)) + (torch.cat([r[3] for r in rows]),)
+        nh, act, arch = self.spec.ids()
+        nll = torch.empty(g, dtype=torch.float64, device=dev)
+        mean = torch.empty((g, self.t), dtype=torch.float64, device=dev)
+        var = torch.empty((g, self.t), dtype=torch.float64, device=dev)
+        info = torch.empty(g, dtype=torch.int32, device=dev)
+        # every slot a CTA the device keeps resident (test_nll_batch_kernel: two per SM), as far as half the free
+        # memory holds them; more slots would only wait
+        one = self.lib.smnngp_test_nll_batch_workspace_bytes(self.n, self.t, nh, arch, 1)
+        with torch.cuda.device(dev):
+            free = torch.cuda.mem_get_info(dev)[0]
+        slots = max(1, min(g, 2 * torch.cuda.get_device_properties(dev).multi_processor_count, free // 2 // one))
+        ws_bytes = slots * one
+        with torch.cuda.device(dev):
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            rc = self.lib.smnngp_test_nll_batch_f64(_stream(dev), _p(self.k0dd), self.ld0, _p(self.k0td), self.ld0,
+                                                    _p(self.q_d), _p(self.q_t), _p(self.y), _p(yt), self.n, self.t, g,
+                                                    nh, act, arch, _p(hps), KIND[kind], float(y_mean), float(y_std),
+                                                    _p(ws), ws_bytes, _p(nll), _p(mean), _p(var), C.c_void_p(0),
+                                                    _p(info))
+        _lib.check(rc, "test_nll_batch")
+        return nll, mean, var, info
 
 
     def sweep_eps(self, eps_list, hp, group=None):

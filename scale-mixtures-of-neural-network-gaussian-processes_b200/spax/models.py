@@ -209,10 +209,15 @@ class MultiStartSPR:
         return out[:, 1], g, info
 
     def test_nll(self, x, y):
-        """[R] SPR.test_nll of every restart (one fused call per restart)."""
+        """[R] SPR.test_nll of every restart.  Where one launch for every restart is faster (``device._batch_wins``,
+        never for N > 4096) the bases of (x_data, x) are computed once and ``GridSearch.test_nll`` evaluates all the
+        restarts in one smnngp_test_nll_batch_f64 launch; elsewhere one fused call per restart."""
         x = torch.as_tensor(x, dtype=torch.float64, device=self.x_data.device)
         y = torch.as_tensor(y, dtype=torch.float64, device=self.x_data.device)
         hps = self.safe_values()
+        if _dev._batch_wins(self.num_data, hps.shape[0]):
+            gs = _dev.GridSearch(self.x_data, self.y_data, x, spec=self.spec)
+            return gs.test_nll(hps, y, self.y_mean, self.y_std, self.kind)[0]
         rows = [_dev.test_nll(self.x_data, self.y_data, x, y, self.y_mean, self.y_std, spec=self.spec, hp=hps[r],
                               kind=self.kind)[0] for r in range(hps.shape[0])]
         return torch.stack(rows)
