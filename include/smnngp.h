@@ -198,7 +198,11 @@ int smnngp_test_nll_batch_f64(void* stream, const double* K0dd, int64_t ld0, con
  *   sample_f_iid : materialises out [C, T, S]
  *   draw_metrics : the same draws, never written: per-point log-likelihood of the true label
  *                  logsumexp_s(log_softmax_c f)[label] - log S  (spax/utils.py:61-66), predicted class
- *                  argmax_c logsumexp_s log_softmax (spax/utils.py:69-74); out_dev[2] = { nll, correct count } */
+ *                  argmax_c logsumexp_s log_softmax (spax/utils.py:69-74); out_dev[2] = { nll, correct count }.
+ *                  A label outside [0, C) gives ll_per_test = NaN (so nll = NaN) and never counts as correct.
+ * Both draw the same value for the same (seed, s, t, c) and launch on the device of `stream`.  T, C or S < 1,
+ * T or S > INT32_MAX, for sample_f_iid C > INT32_MAX or C * T * S > INT64_MAX, for draw_metrics C > 16, an invalid
+ * kind or a null pointer: SMNNGP_EINVAL before anything is enqueued, with smnngp_last_error() naming the call. */
 int smnngp_sample_f_iid_f64(void* stream, const double* mean, const double* var, int var_per_class, int64_t T,
                             int64_t C, int64_t S, const double* hp_dev, int kind, uint64_t seed, double* out);
 int smnngp_draw_metrics_f64(void* stream, const double* mean, const double* var, int var_per_class,

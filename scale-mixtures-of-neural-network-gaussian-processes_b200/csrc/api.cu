@@ -762,6 +762,33 @@ int smnngp_test_nll_batch_f64(void* stream, const double* K0dd, int64_t ld0, con
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// posterior draw stage (draws.cu)
+// ---------------------------------------------------------------------------------------------------------
+int smnngp_sample_f_iid_f64(void* stream, const double* mean, const double* var, int var_per_class, int64_t T,
+                            int64_t C, int64_t S, const double* hp_dev, int kind, uint64_t seed, double* out) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  if (!mean || !var || !hp_dev || !out || T <= 0 || C <= 0 || S <= 0 || T > INT32_MAX || C > INT32_MAX ||
+      S > INT32_MAX || C * T > INT64_MAX / S || (kind != KIND_GAUSS && kind != KIND_STUDENT_T))
+    return fail(SMNNGP_EINVAL, "smnngp_sample_f_iid_f64: invalid argument");
+  CU(launch_sample_f_iid(s, mean, var, var_per_class, (int)T, (int)C, (int)S, hp_dev, kind, seed, out));
+  return SMNNGP_OK;
+}
+
+int smnngp_draw_metrics_f64(void* stream, const double* mean, const double* var, int var_per_class,
+                            const int* label, int64_t T, int64_t C, int64_t S, const double* hp_dev, int kind,
+                            uint64_t seed, double* ll_per_test, int* pred, double* out_dev) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  if (!mean || !var || !label || !hp_dev || !ll_per_test || !pred || !out_dev || T <= 0 || C <= 0 || C > DRAW_MAXC ||
+      S <= 0 || T > INT32_MAX || S > INT32_MAX || (kind != KIND_GAUSS && kind != KIND_STUDENT_T))
+    return fail(SMNNGP_EINVAL, "smnngp_draw_metrics_f64: invalid argument");
+  CU(launch_draw_metrics(s, mean, var, var_per_class, label, (int)T, (int)C, (int)S, hp_dev, kind, seed, ll_per_test,
+                         pred, out_dev));
+  return SMNNGP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // host-buffer entry points
 // ---------------------------------------------------------------------------------------------------------
 void smnngp_host_release(void) {

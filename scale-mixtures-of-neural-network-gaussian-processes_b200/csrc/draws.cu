@@ -7,14 +7,11 @@
 // so that for S = 10^4 draws x T = 10^4 points x C = 10 classes nothing but the T results ever touches HBM.
 // Because the generator is counter based the fused kernel sees exactly the draws the materialising one writes,
 // which is what the parity test relies on.  (Bit parity with JAX's threefry stream is not a goal.)
-#include "../../include/smnngp.h"
 #include "kernels.cuh"
 
-using namespace smnngp;
+namespace smnngp {
 
 namespace {
-
-constexpr int DRAW_MAXC = 16;
 
 struct Philox {
   uint32_t k0, k1;
@@ -155,7 +152,7 @@ draw_metrics_kernel(const double* __restrict__ mean, const double* __restrict__ 
       if (c < C) acc[c].add(f[c] - lse);
   }
   // fixed-order merge over the block, one class at a time
-  double best = -INFINITY, ll_true = 0.0;
+  double best = -INFINITY, ll_true = __longlong_as_double(0x7ff8000000000000ll);   // stays NaN if y is not in [0, C)
   int best_c = 0;
   for (int c = 0; c < C; c++) {
     double m = -INFINITY, s = 0.0;
@@ -206,35 +203,28 @@ __global__ void draw_finalize_kernel(const double* __restrict__ ll_per_test, con
 
 }  // namespace
 
-extern "C" {
-
-int smnngp_sample_f_iid_f64(void* stream, const double* mean, const double* var, int var_per_class, int64_t T,
-                            int64_t C, int64_t S, const double* hp_dev, int kind, uint64_t seed, double* out) {
-  if (!mean || !var || !hp_dev || !out || T <= 0 || C <= 0 || S <= 0 || (kind != KIND_GAUSS && kind != KIND_STUDENT_T))
-    return SMNNGP_EINVAL;
+cudaError_t launch_sample_f_iid(cudaStream_t s, const double* mean, const double* var, int var_per_class, int T, int C,
+                                int S, const double* hp, int kind, uint64_t seed, double* out) {
   const long long total = (long long)C * T * S;
   long long blocks = (total + 255) / 256;
   if (blocks > 148 * 16) blocks = 148 * 16;
-  sample_f_iid_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      mean, var, var_per_class, (int)T, (int)C, (int)S, hp_dev, kind, (uint32_t)seed, (uint32_t)(seed >> 32), out);
+  sample_f_iid_kernel<<<(unsigned)blocks, 256, 0, s>>>(mean, var, var_per_class, T, C, S, hp, kind, (uint32_t)seed,
+                                                       (uint32_t)(seed >> 32), out);
   instr().launches++;
-  return cudaGetLastError() == cudaSuccess ? SMNNGP_OK : SMNNGP_ECUDA;
+  return cudaGetLastError();
 }
 
-int smnngp_draw_metrics_f64(void* stream, const double* mean, const double* var, int var_per_class,
-                            const int* label, int64_t T, int64_t C, int64_t S, const double* hp_dev, int kind,
-                            uint64_t seed, double* ll_per_test, int* pred, double* out_dev) {
-  if (!mean || !var || !label || !hp_dev || !ll_per_test || !pred || !out_dev || T <= 0 || C <= 0 || C > DRAW_MAXC ||
-      S <= 0 || (kind != KIND_GAUSS && kind != KIND_STUDENT_T))
-    return SMNNGP_EINVAL;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  draw_metrics_kernel<<<(unsigned)T, 256, 0, s>>>(mean, var, var_per_class, label, (int)T, (int)C, (int)S, hp_dev, kind,
-                                                  (uint32_t)seed, (uint32_t)(seed >> 32), ll_per_test, pred);
+cudaError_t launch_draw_metrics(cudaStream_t s, const double* mean, const double* var, int var_per_class,
+                                const int* label, int T, int C, int S, const double* hp, int kind, uint64_t seed,
+                                double* ll_per_test, int* pred, double* out) {
+  draw_metrics_kernel<<<(unsigned)T, 256, 0, s>>>(mean, var, var_per_class, label, T, C, S, hp, kind, (uint32_t)seed,
+                                                  (uint32_t)(seed >> 32), ll_per_test, pred);
   instr().launches++;
-  if (cudaGetLastError() != cudaSuccess) return SMNNGP_ECUDA;
-  draw_finalize_kernel<<<1, 1024, 0, s>>>(ll_per_test, pred, label, (int)T, out_dev);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  draw_finalize_kernel<<<1, 1024, 0, s>>>(ll_per_test, pred, label, T, out);
   instr().launches++;
-  return cudaGetLastError() == cudaSuccess ? SMNNGP_OK : SMNNGP_ECUDA;
+  return cudaGetLastError();
 }
 
-}  // extern "C"
+}  // namespace smnngp

@@ -185,6 +185,16 @@ struct TestNllBatchParams {
 // one persistent launch: min(slots, G) CTAs, each owns one slot and evaluates points blockIdx.x, + gridDim.x, ...
 cudaError_t launch_test_nll_batch(cudaStream_t s, const TestNllBatchParams& p, int act, long long slots);
 
+// ---- posterior draw stage (draws.cu) -------------------------------------------------------------------------
+constexpr int DRAW_MAXC = 16;   // classes draw_metrics keeps in registers
+// out [C, T, S] <- mean [T, C] + sigma [C, T] * variate, one counter-based Philox stream per (s, t, c)
+cudaError_t launch_sample_f_iid(cudaStream_t s, const double* mean, const double* var, int var_per_class, int T, int C,
+                                int S, const double* hp, int kind, uint64_t seed, double* out);
+// the same draws, reduced to ll_per_test [T], pred [T] and out [2] = { nll, correct count }; C <= DRAW_MAXC
+cudaError_t launch_draw_metrics(cudaStream_t s, const double* mean, const double* var, int var_per_class,
+                                const int* label, int T, int C, int S, const double* hp, int kind, uint64_t seed,
+                                double* ll_per_test, int* pred, double* out);
+
 // ---- gradient of the log marginal likelihood (grad.cu) -------------------------------------------------------
 // tab3 [3][n_act][tab_ld]: encoded marginal variances + the two dual planes the gradient epilogue needs
 cudaError_t launch_qtable_dual(cudaStream_t s, const double* X, long long ldx, int N, int D, int n_hidden, int act,
