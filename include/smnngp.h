@@ -130,7 +130,7 @@ int smnngp_test_nll_f64(void* stream, const double* X, const double* y, const do
  *   grid_point  one grid point from the bases: recursion-only passes (8 B read + 8 B written per entry) + the two
  *               factorisations.  mean_out [T], var_out [T] (predict(eps), relative regulariser);
  *               out_dev[2] = { sum log L_ii of chol(K + eps I)  (= 1/2 log det),  y^T (K + eps I)^-1 y }.
- * The (alpha, beta) importance-sampling table that follows (find.py:163-186) is host arithmetic on these outputs. */
+ * The importance-sampling table that follows (find.py:163-191) is smnngp_mixture_nll_f64 on these outputs. */
 int smnngp_grid_base_f64(void* stream, const double* X, const double* Xt, int64_t N, int64_t T, int64_t D,
                          double* K0dd, int64_t ld0, double* K0td, int64_t ld0t, double* q_d, double* q_t);
 size_t smnngp_grid_workspace_bytes(int64_t N, int64_t T, int n_hidden, int arch);
@@ -208,6 +208,39 @@ int smnngp_sample_f_iid_f64(void* stream, const double* mean, const double* var,
 int smnngp_draw_metrics_f64(void* stream, const double* mean, const double* var, int var_per_class,
                             const int* label, int64_t T, int64_t C, int64_t S, const double* hp_dev, int kind,
                             uint64_t seed, double* ll_per_test, int* pred, double* out_dev);
+
+/* ---- scale mixture by importance sampling: the reference's table over prior parameters at the end of its grid search
+ * (experiments/regression/find.py:163-191), for a prior on the output scale with no conjugate form.  A scale s > 0
+ * multiplies the whole covariance, y | s ~ N(0, s A) with A = K + eps I, f_t | y, s ~ N(m_t, s v_t) with the
+ * predictive of the relative regulariser.  For draws s_1 .. s_S of the prior,
+ *   l_j    = -(N/2) log s_j - quad / (2 s_j)          (-inf for s_j = 0 or +inf: zero weight, never NaN)
+ *   lml    = logsumexp_j l_j - log S - sum log L_ii - (N/2) log 2 pi
+ *   logp_t = logsumexp_j [l_j + log N(y~_t; m~_t, s_j v~_t)] - logsumexp_j l_j, de-standardised as test_nll:
+ *            y~ = yt y_std + y_mean, m~ = m y_std + y_mean, v~ = v y_std^2
+ *   nll    = -mean_t logp_t,  ess = (sum_j w_j)^2 / sum_j w_j^2 with w_j = exp(l_j - max l).
+ * If every l_j = -inf: ess = 0, lml = -inf, nll and logp NaN.  A NaN in scal[g] makes every output of row g NaN; a
+ * NaN draw makes every output of its row p NaN.
+ *   scale_draws  draws_out [P][S] from the prior of row p, params_dev [P][2]: INVGAMMA (a, b), s = b / Gamma(a);
+ *                BURR12 (c, k), CDF 1 - (1 + s^c)^-k, s = exp(log(expm1(-log u / k)) / c) from one 53-bit u in (0, 1].
+ *                Philox4x32-10 keyed by seed, counter (j, p, 0xFFFFFFFF, n), a stream the posterior draws never use;
+ *                the draws do not depend on the grid point, so every point sees the same draws.  A row whose
+ *                parameters are <= 0 or not finite gives NaN draws.
+ *   mixture_nll  every (g, p) pair in one launch: scal [G][2] = out_dev of grid_point / grid_batch (or out[2], out[3]
+ *                of smnngp_lml_f64 with kind = gauss), mean / var [G][ld] (row g: that point's predictive), yt [T],
+ *                draws [P][S] (scale_draws or the caller's own).  lml_out, ess_out and nll_out are [G][P], logp_out
+ *                [G][P][T] or NULL.  T = 0 is the evidence alone: mean, var, yt, nll_out and logp_out may then be NULL.
+ *                A pair's outputs are the same bits in any G, P or order, with or without logp_out.
+ * N, G, P or S < 1, T < 0, ld < T, an invalid family, y_std <= 0 or not finite, a null required pointer, an index
+ * product beyond int64, for scale_draws P or S > INT32_MAX: SMNNGP_EINVAL before anything is enqueued, with
+ * smnngp_last_error() naming the call.  Each call launches on the device of `stream`, is one kernel launch, allocates
+ * nothing and is graph-capturable. */
+enum { SMNNGP_SCALE_INVGAMMA = 0, SMNNGP_SCALE_BURR12 = 1 };
+int smnngp_scale_draws_f64(void* stream, int family, const double* params_dev, int64_t P, int64_t S, uint64_t seed,
+                           double* draws_out);
+int smnngp_mixture_nll_f64(void* stream, const double* scal, const double* mean, const double* var, int64_t ld,
+                           const double* yt, int64_t N, int64_t T, int64_t G, const double* draws, int64_t P,
+                           int64_t S, double y_mean, double y_std, double* nll_out, double* lml_out, double* ess_out,
+                           double* logp_out);
 
 /* ---- stage-level entry points (multi-GPU driver: one process per GPU interleaves these with NCCL collectives;
  * same kernels as the fused calls).  Layout and algorithm: DESIGN.md section 7.

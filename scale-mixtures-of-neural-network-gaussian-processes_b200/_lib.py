@@ -16,7 +16,7 @@ LIB_DIR = os.path.join(_HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libsmnngp.so")
 SOURCES = ["gram.cu", "chol.cu", "reduce.cu", "api.cu", "stages.cu", "draws.cu", "grad.cu", "peer.cu", "exchange.cu",
            "context.cu", "trtri.cu", "multigpu.cu", "grid_batch.cu",
-           "grad_batch.cu", "test_nll_batch.cu"]
+           "grad_batch.cu", "test_nll_batch.cu", "mixture.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Wno-deprecated-gpu-targets"]
 
@@ -33,6 +33,7 @@ EXPORTS = [
     "smnngp_grid_batch_workspace_bytes", "smnngp_grid_batch_f64",
     "smnngp_lml_grad_batch_workspace_bytes", "smnngp_lml_grad_batch_f64",
     "smnngp_test_nll_batch_workspace_bytes", "smnngp_test_nll_batch_f64",
+    "smnngp_scale_draws_f64", "smnngp_mixture_nll_f64",
     "smnngp_stage_qtable_f64", "smnngp_stage_gram_f64", "smnngp_stage_factor_diag_f64", "smnngp_stage_trsm_f64",
     "smnngp_stage_update_f64", "smnngp_stage_sumsq_f64", "smnngp_stage_lml_finalize_f64",
     "smnngp_stage_predict_finalize_f64", "smnngp_stage_test_nll_finalize_f64",
@@ -208,6 +209,9 @@ def _declare(lib):
     lib.smnngp_test_nll_batch_workspace_bytes.argtypes = [_i64, _i64, _i, _i, _i64]
     lib.smnngp_test_nll_batch_f64.argtypes = [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i, _i,
                                               _i, _vp, _i, _d, _d, _vp, _sz, _vp, _vp, _vp, _vp, _vp]
+    lib.smnngp_scale_draws_f64.argtypes = [_vp, _i, _vp, _i64, _i64, C.c_uint64, _vp]
+    lib.smnngp_mixture_nll_f64.argtypes = [_vp, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _i64, _i64, _d, _d,
+                                           _vp, _vp, _vp, _vp]
     lib.smnngp_sample_f_iid_f64.argtypes = [_vp, _vp, _vp, _i, _i64, _i64, _i64, _vp, _i, C.c_uint64, _vp]
     lib.smnngp_draw_metrics_f64.argtypes = [_vp, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _i, C.c_uint64, _vp, _vp, _vp]
     lib.smnngp_stage_qtable_f64.argtypes = [_vp, _vp, _i64, _i64, _i, _i, _i, _vp, _vp, _i64, _vp, _vp]

@@ -789,6 +789,52 @@ int smnngp_draw_metrics_f64(void* stream, const double* mean, const double* var,
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// scale mixture by importance sampling (mixture.cu)
+// ---------------------------------------------------------------------------------------------------------
+namespace {
+// a * b for a, b >= 0, false when it does not fit an int64
+bool mul_ok(int64_t a, int64_t b, int64_t* out) {
+  if (a != 0 && b > INT64_MAX / a) return false;
+  *out = a * b;
+  return true;
+}
+}  // namespace
+
+int smnngp_scale_draws_f64(void* stream, int family, const double* params_dev, int64_t P, int64_t S, uint64_t seed,
+                           double* draws_out) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  int64_t PS = 0;
+  // P and S are Philox counter words (32 bits)
+  if (!params_dev || !draws_out || P < 1 || S < 1 || P > INT32_MAX || S > INT32_MAX || !mul_ok(P, S, &PS) ||
+      (family != SCALE_INVGAMMA && family != SCALE_BURR12))
+    return fail(SMNNGP_EINVAL, "smnngp_scale_draws_f64: invalid argument");
+  CU(launch_scale_draws(s, family, params_dev, P, S, seed, draws_out));
+  return SMNNGP_OK;
+}
+
+int smnngp_mixture_nll_f64(void* stream, const double* scal, const double* mean, const double* var, int64_t ld,
+                           const double* yt, int64_t N, int64_t T, int64_t G, const double* draws, int64_t P,
+                           int64_t S, double y_mean, double y_std, double* nll_out, double* lml_out, double* ess_out,
+                           double* logp_out) {
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  Enter scope(s);
+  int64_t GP = 0, PS = 0, GPT = 0, Gld = 0;
+  const bool tests_ok = T == 0 || (mean && var && yt && nll_out);
+  if (!scal || !draws || !lml_out || !ess_out || !tests_ok || N < 1 || T < 0 || G < 1 || P < 1 || S < 1 || ld < T ||
+      !(y_std > 0.0) || !(y_std < INFINITY) || !mul_ok(G, P, &GP) || !mul_ok(P, S, &PS) || !mul_ok(GP, T, &GPT) ||
+      !mul_ok(G, ld, &Gld))
+    return fail(SMNNGP_EINVAL, "smnngp_mixture_nll_f64: invalid argument");
+  MixtureParams p{};
+  p.scal = scal; p.mean = mean; p.var = var; p.yt = yt; p.draws = draws;
+  p.N = N; p.T = T; p.G = G; p.P = P; p.S = S; p.ld = ld;
+  p.y_mean = y_mean; p.y_std = y_std;
+  p.nll = nll_out; p.lml = lml_out; p.ess = ess_out; p.logp = logp_out;
+  CU(launch_mixture_nll(s, p));
+  return SMNNGP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // host-buffer entry points
 // ---------------------------------------------------------------------------------------------------------
 void smnngp_host_release(void) {

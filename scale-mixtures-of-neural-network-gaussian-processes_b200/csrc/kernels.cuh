@@ -195,6 +195,24 @@ cudaError_t launch_draw_metrics(cudaStream_t s, const double* mean, const double
                                 const int* label, int T, int C, int S, const double* hp, int kind, uint64_t seed,
                                 double* ll_per_test, int* pred, double* out);
 
+// ---- scale mixture by importance sampling (mixture.cu) --------------------------------------------------------
+enum ScaleFamily { SCALE_INVGAMMA = 0, SCALE_BURR12 = 1 };
+// draws [P][S] of the scale prior of row p (params [P][2]: (a, b) or (c, k)); counter (j, p, 0xFFFFFFFF, n)
+cudaError_t launch_scale_draws(cudaStream_t s, int family, const double* params, long long P, long long S,
+                               uint64_t seed, double* out);
+struct MixtureParams {
+  const double* scal;                          // [G][2] {sum log L_ii, y^T A^-1 y}
+  const double *mean, *var;                    // [G][ld] predictive (standardised units); null when T = 0
+  const double* yt;                            // [T] standardised test targets
+  const double* draws;                         // [P][S]
+  long long N, T, G, P, S, ld;
+  double y_mean, y_std;
+  double *nll, *lml, *ess;                     // [G][P]; nll may be null when T = 0
+  double* logp;                                // [G][P][T] or null
+};
+// one launch, a warp per (g, p) pair; a pair's outputs depend only on its rows and the scalars
+cudaError_t launch_mixture_nll(cudaStream_t s, const MixtureParams& p);
+
 // ---- gradient of the log marginal likelihood (grad.cu) -------------------------------------------------------
 // tab3 [3][n_act][tab_ld]: encoded marginal variances + the two dual planes the gradient epilogue needs
 cudaError_t launch_qtable_dual(cudaStream_t s, const double* X, long long ldx, int N, int D, int n_hidden, int act,

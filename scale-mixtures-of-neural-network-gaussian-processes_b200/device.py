@@ -396,8 +396,8 @@ def grid_point(x, y, x_test, *, spec: StackSpec, hp):
     """The device work of ONE point (w_std, b_std, eps) of the reference's grid search
     (experiments/regression/find.py:134-160): the predictive with the RELATIVE regulariser (``predict(eps)``,
     find.py:75-77) and, for the absolute one, ``log det(K + eps I)`` and ``y^T (K + eps I)^-1 y``
-    (find.py:149-156, there through an explicit inverse and ``multivariate_normal.logpdf``).  The (alpha, beta)
-    importance-sampling table that follows (find.py:163-186) is host arithmetic on these outputs.
+    (find.py:149-156, there through an explicit inverse and ``multivariate_normal.logpdf``).  The importance-sampling
+    table that follows (find.py:163-191) is ``GridSearch.mixture``.
     Returns (mean [T], var [T], logdet, quad, info) with logdet = log det(K + eps I)."""
     mean, var, info1 = predict(x, y, x_test, spec=spec, hp=hp, shift="eps_rel")
     out, info2 = lml(x, y, spec=spec, hp=hp, kind="gauss")
@@ -536,6 +536,20 @@ class GridSearch:
         return nll, mean, var, info
 
 
+    def mixture(self, hps, y_test, y_mean, y_std, *, family, params, num_samples=1000, seed=0):
+        """The importance-sampling table at the end of the reference's grid search (find.py:163-191): for every row of
+        ``hps`` [G, 6] (grid points) and every row of ``params`` [P, 2] (prior parameters of ``family``, see
+        ``scale_draws``), the evidence and test NLL of the scale mixture over ``num_samples`` prior draws.  One
+        ``points(hps)`` call (batched or looped, so any N), one draw launch and one mixture launch; every grid point sees
+        the same draws.  Returns (nll [G, P], lml [G, P], ess [G, P])."""
+        dev = self.y.device
+        mean, var, logdet, quad, _ = self.points(hps)
+        scal = torch.stack([0.5 * logdet, quad], dim=1)
+        with torch.cuda.device(dev):
+            draws = scale_draws(family, _f64(params, dev), num_samples, seed=seed)
+            nll, lml, ess, _ = mixture_nll(scal, mean, var, y_test, self.n, draws, y_mean, y_std)
+        return nll, lml, ess
+
     def sweep_eps(self, eps_list, hp, group=None):
         """find.py:141 `for eps in eps_list`: every regulariser of the sweep for the scalars in ``hp`` (its eps entry is
         replaced), one epsilon per GPU when a process group is up (replica parallelism, see distributed.sweep_eps)."""
@@ -653,3 +667,60 @@ def draw_metrics(mean, var, label, *, hp, kind="student_t", num_samples, seed=0)
                                      c, int(num_samples), _p(hp), KIND[kind], int(seed), _p(ll), _p(pred), _p(out))
     _lib.check(rc, "draw_metrics")
     return out[0], out[1], ll, pred
+
+
+# ---------------------------------------------------------------------------------------------------------
+# scale mixture by importance sampling (a prior on the output scale without a conjugate form)
+SCALE_FAMILY = {"invgamma": 0, "burr12": 1}
+
+
+def scale_draws(family, params, num_samples, seed=0):
+    """[P, S] draws of the scale prior of every row of ``params`` [P, 2] (device): ``"invgamma"`` (a, b), s = b /
+    Gamma(a); ``"burr12"`` (c, k), CDF 1 - (1 + s^c)^-k.  Counter-based: draw (p, j) depends only on (seed, p, j)."""
+    _require_cuda()
+    if family not in SCALE_FAMILY:
+        raise ValueError(f"unknown scale family '{family}'")
+    lib = _lib.load()
+    params = _f64(params)
+    if params.ndim != 2 or params.shape[1] != 2:
+        raise ValueError("params must be [P, 2]")
+    out = torch.empty((params.shape[0], int(num_samples)), dtype=torch.float64, device=params.device)
+    with torch.cuda.device(params.device):
+        rc = lib.smnngp_scale_draws_f64(_stream(params.device), SCALE_FAMILY[family], _p(params), params.shape[0],
+                                        int(num_samples), int(seed) & 0xFFFFFFFFFFFFFFFF, _p(out))
+    _lib.check(rc, "scale_draws")
+    return out
+
+
+@_on_device_of_first_arg
+def mixture_nll(scal, mean, var, y_test, n, draws, y_mean, y_std, logp=False):
+    """The scale mixture at every (grid point g, draw row p) pair in one launch (include/smnngp.h,
+    smnngp_mixture_nll_f64): ``scal`` [G, 2] = {sum log L_ii, y^T A^-1 y} of A = K + eps I, ``mean`` / ``var`` [G, T]
+    the predictive (relative regulariser, standardised units), ``y_test`` [T] standardised, ``n`` training rows,
+    ``draws`` [P, S] scales.  T = 0 (mean, var, y_test None) is the evidence alone.  Returns (nll [G, P], lml [G, P],
+    ess [G, P], logp [G, P, T] or None); nll is None when T = 0."""
+    _require_cuda()
+    lib = _lib.load()
+    scal = _f64(scal)
+    dev = scal.device
+    draws = _f64(draws, dev)
+    if scal.ndim != 2 or scal.shape[1] != 2 or draws.ndim != 2:
+        raise ValueError("scal must be [G, 2] and draws [P, S]")
+    g, (p, s) = scal.shape[0], draws.shape
+    if y_test is None:
+        t = 0
+        mean = var = yt = nll = lp = None
+    else:
+        yt = _f64(y_test, dev)
+        t = yt.shape[0]
+        mean, var = _f64(mean, dev), _f64(var, dev)
+        if tuple(mean.shape) != (g, t) or tuple(var.shape) != (g, t):
+            raise ValueError(f"mean and var must be [{g}, {t}]")
+        nll = torch.empty((g, p), dtype=torch.float64, device=dev)
+        lp = torch.empty((g, p, t), dtype=torch.float64, device=dev) if logp else None
+    lml = torch.empty((g, p), dtype=torch.float64, device=dev)
+    ess = torch.empty((g, p), dtype=torch.float64, device=dev)
+    rc = lib.smnngp_mixture_nll_f64(_stream(dev), _p(scal), _p(mean), _p(var), t, _p(yt), int(n), t, g, _p(draws),
+                                    p, s, float(y_mean), float(y_std), _p(nll), _p(lml), _p(ess), _p(lp))
+    _lib.check(rc, "mixture_nll")
+    return nll, lml, ess, lp

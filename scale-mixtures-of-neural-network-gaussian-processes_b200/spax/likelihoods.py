@@ -8,7 +8,7 @@ from .bijectors import positive
 from .utils import multivariate_t_logpdf, multivariate_normal_logpdf
 from .. import device as _dev
 
-__all__ = ["Likelihood", "GaussianLikelihood", "StudentTLikelihood"]
+__all__ = ["Likelihood", "GaussianLikelihood", "StudentTLikelihood", "BurrXIILikelihood"]
 
 
 def _diag(cov):
@@ -58,3 +58,23 @@ class StudentTLikelihood(Likelihood):
         norm = (math.lgamma(cond_df / 2) + 0.5 * math.log(cond_df) + 0.5 * torch.log(sigma * sigma * math.pi)
                 - math.lgamma((cond_df + 1) / 2))
         return -(norm + (cond_df + 1) / 2 * torch.log1p(z * z / cond_df))
+
+
+class BurrXIILikelihood(Likelihood):
+    """Scale mixture of NNGPs with a Burr Type XII prior on the output scale (CDF 1 - (1 + s^c)^-k): y | s ~ N(0, s A).
+    The prior has no conjugate form, so ``SPR.loss`` and ``SPR.test_nll`` importance-sample the scale over
+    ``num_samples`` prior draws (``device.scale_draws`` with a fixed ``seed``: every evaluation sees the same draws).
+    Only the fused path of an smnngp ``KernelFn`` evaluates it, and there is no gradient."""
+    require = None
+    kind = "burr12"
+
+    def __init__(self, c, k, *, num_samples=1000, seed=0):
+        self.c = ConstraintTrainVar(c, constraint=positive())
+        self.k = ConstraintTrainVar(k, constraint=positive())
+        self.num_samples = int(num_samples)
+        self.seed = int(seed)
+
+    def draws(self, device):
+        """[1, num_samples] scale draws of the current (c, k)"""
+        params = torch.tensor([[self.c.safe_value, self.k.safe_value]], dtype=torch.float64, device=device)
+        return _dev.scale_draws("burr12", params, self.num_samples, seed=self.seed)

@@ -34,8 +34,30 @@ class SPR(Module):
     def _fused(self, kernel_fn):
         return isinstance(kernel_fn, KernelFn) and getattr(self.likelihood, "kind", None) in _dev.KIND
 
+    def _mixture(self, kernel_fn):
+        """Whether the likelihood is an importance-sampled scale mixture (BurrXIILikelihood); it needs the fused path"""
+        if getattr(self.likelihood, "kind", None) != "burr12":
+            return False
+        if not isinstance(kernel_fn, KernelFn):
+            raise TypeError("BurrXIILikelihood needs a kernel_fn built by smnngp nt_kernels")
+        return True
+
+    def _mixture_pieces(self, kernel_fn):
+        """(x, y, hp, scal [1, 2], draws [1, S]) on the device: {sum log L_ii, y^T A^-1 y} of A = K + eps I from the
+        Gaussian LML and the likelihood's scale draws"""
+        x = _dev._f64(self.x_data, "cuda" if not isinstance(self.x_data, torch.Tensor) else None)
+        y = _dev._f64(self.y_data, x.device)
+        hp = kernel_fn.hp(x.device, **self._hp_args())
+        out, _ = _dev.lml(x, y, spec=kernel_fn.spec, hp=hp, kind="gauss")
+        return x, y, hp, out[2:4].reshape(1, 2), self.likelihood.draws(x.device)
+
     def loss(self):
         kernel_fn = self.kernel.get_kernel_fn()
+        if self._mixture(kernel_fn):
+            x, _, _, scal, draws = self._mixture_pieces(kernel_fn)
+            _, lml, _, _ = _dev.mixture_nll(scal, None, None, None, self.num_data, draws, 0.0, 1.0)
+            loss = -lml[0, 0] / self.num_data
+            return float(loss) if isinstance(self.x_data, np.ndarray) else loss
         if self._fused(kernel_fn):
             host = isinstance(self.x_data, np.ndarray)
             hp = kernel_fn.hp_host(**self._hp_args()) if host else kernel_fn.hp(self.x_data.device, **self._hp_args())
@@ -53,6 +75,8 @@ class SPR(Module):
         (spax/base.py:23-25, spax/bijectors.py:51-53) is applied here.  Scalars the likelihood does not own
         (Gaussian: alpha, beta) are absent."""
         kernel_fn = self.kernel.get_kernel_fn()
+        if getattr(self.likelihood, "kind", None) == "burr12":
+            raise TypeError("loss_and_grad: the importance-sampled scale mixture (BurrXIILikelihood) has no gradient")
         if not self._fused(kernel_fn):
             raise TypeError("loss_and_grad needs a kernel_fn built by smnngp nt_kernels and a spax likelihood")
         host = isinstance(self.x_data, np.ndarray)
@@ -70,6 +94,13 @@ class SPR(Module):
 
     def test_nll(self, x, y):
         kernel_fn = self.kernel.get_kernel_fn()
+        if self._mixture(kernel_fn):
+            xd, yd, hp, scal, draws = self._mixture_pieces(kernel_fn)
+            xt, yt = _dev._f64(x, xd.device), _dev._f64(y, xd.device)
+            mean, var, _ = _dev.predict(xd, yd, xt, spec=kernel_fn.spec, hp=hp, shift="eps_rel")
+            nll, _, _, _ = _dev.mixture_nll(scal, mean.reshape(1, -1), var.reshape(1, -1), yt, self.num_data, draws,
+                                            float(self.y_mean), float(self.y_std))
+            return float(nll[0, 0]) if isinstance(self.x_data, np.ndarray) else nll[0, 0]
         if self._fused(kernel_fn):
             host = isinstance(self.x_data, np.ndarray)
             hp = kernel_fn.hp_host(**self._hp_args()) if host else kernel_fn.hp(self.x_data.device, **self._hp_args())
@@ -173,6 +204,8 @@ class MultiStartSPR:
 
     def __init__(self, kernel, likelihood, x_data, y_data, y_mean, y_std, *, starts):
         kernel_fn = kernel.get_kernel_fn()
+        if getattr(likelihood, "kind", None) == "burr12":
+            raise TypeError("MultiStartSPR: the importance-sampled scale mixture (BurrXIILikelihood) has no gradient")
         if not (isinstance(kernel_fn, KernelFn) and getattr(likelihood, "kind", None) in _dev.KIND):
             raise TypeError("MultiStartSPR needs a kernel_fn built by smnngp nt_kernels and a spax likelihood")
         self.spec, self.kind = kernel_fn.spec, likelihood.kind
